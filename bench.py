@@ -25,6 +25,8 @@ import subprocess
 import sys
 import time
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -63,7 +65,47 @@ def parse_args():
     ap.add_argument("--no-dist-commit", action="store_true", help="N>1: skip the one-commitment-over-all-ranks measurements")
     ap.add_argument("--no-prove", action="store_true", help="skip the end-to-end shard-prove timings (BASELINE configs 1-3)")
     ap.add_argument("--no-e2e", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed commit returned (root, a fixed sample of opened LDE rows "
+                         "with their Merkle paths) as DIR/<name>.npy in float64, to compare two builds output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+# cap of everything --dump-outputs writes; the sample below stays far under it at the default size
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_ROWS = 2048  # opened LDE rows (and their Merkle paths) in the dump, at fixed pseudo-random indices
+
+
+def dump_outputs(out_dir, arrays):
+    """Write {name: array} as out_dir/<name>.npy in float64 (every u32 field element is exact there)."""
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"bench.py: --dump-outputs would write {total} bytes, more than {DUMP_LIMIT_BYTES}")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+    log(f"bench.py: wrote {', '.join(sorted(arrays))} to {out_dir}")
+
+
+def dump_commit_sample(ctx, bf, handle):
+    """The caller's view of one `Pcs::commit`: its prover data, sampled as Merkle openings (the LDE row at a fixed, seeded
+    set of leaf indices and its authentication path), the way FRI queries read it."""
+    data = bf.PcsProverData(ctx, handle)
+    leaves, cols = data.dims[0]
+    per_row = 8 * (1 + cols + 8 * (leaves.bit_length() - 1))  # float64 bytes of one index, row and path
+    idx = np.sort(np.random.default_rng(0xD0).choice(leaves, size=min(leaves, DUMP_ROWS, DUMP_LIMIT_BYTES // 2 // per_row), replace=False))
+    mmcs = bf.MerkleTreeMmcs(ctx)
+    rows, paths = [], []
+    for i in idx:
+        r, p = mmcs.open_batch(int(i), data.tree)
+        rows.append(r[0])
+        paths.append(p)
+    data.free()
+    return {"opened_row_index": idx, "opened_rows": np.stack(rows), "opening_paths": np.stack(paths)}
 
 
 def workload_name(log_rows, cols):
@@ -375,6 +417,8 @@ def run_reference(args, rank, world):
         "root": r["root"],
         "root_matches_oracle_golden": (r["root"] == golden_root(args.log_rows, args.cols)) if r["full"] and golden_root(args.log_rows, args.cols) else None,
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"commit_root": r["root"]})
     print(json.dumps(line), flush=True)
 
 
@@ -475,14 +519,16 @@ def main():
     if world == 1:
         mat = bf.Mat(trace.data_ptr(), R, W)
 
-        def commit_once():
+        def commit_once(keep=False):
             h = C.c_void_p()
             ctx.check(lib.bfgpu_pcs_commit(ctx._h, C.byref(mat), None, 1, root_p, C.byref(h)))
+            if keep:  # the caller takes the prover data
+                return h
             lib.bfgpu_pcs_data_free(h)
     else:
         shm = shard.ShmComm(dist)  # handles / barrier / caps of every commitment through shared memory instead of NCCL collectives
 
-        def commit_once(src=None):
+        def commit_once(src=None, keep=False):  # every rank holds only its shard of the prover data: the root is the output
             dc = shard.DistributedCommit(ctx, dist, [R], [W], exchange="p2p", comm=shm)
             root[:] = dc.commit([src if src is not None else (trace.data_ptr(), R, nloc)])
             dc.free()
@@ -498,10 +544,11 @@ def main():
     ctx.profile_enable(True)
     launches0 = ctx.launch_count
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    last_data = None
     with torch.cuda.stream(stream):
         ev0.record(stream)
-        for _ in range(args.steps):
-            commit_once()
+        for i in range(args.steps):
+            last_data = commit_once(keep=bool(args.dump_outputs) and i == args.steps - 1)
         ev1.record(stream)
     barrier()
     ms_total = ev0.elapsed_time(ev1)
@@ -510,6 +557,8 @@ def main():
     ctx.profile_enable(False)
     clocks = sampler.stop()
     root_dev = root.copy()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"commit_root": root_dev, **(dump_commit_sample(ctx, bf, last_data) if last_data is not None else {})})
     ms_total = shard.max_over_ranks(ms_total, dist, "cuda")
     ms_step = ms_total / args.steps
     value = algorithmic_bytes(R, W) / (ms_step * 1e-3) / 1e9  # N > 1: the one commitment is the whole job (strong scaling)

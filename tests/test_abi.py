@@ -33,7 +33,9 @@ def test_library_exports_every_declared_symbol():
 
 
 def test_library_is_sm100a_native():
-    out = subprocess.run(["cuobjdump", "-lelf", bf.SO_PATH], capture_output=True, text=True).stdout
+    # the toolkit that built the library (build.py's nvcc), which need not be on PATH
+    cuobjdump = os.path.join(os.path.dirname(os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")), "cuobjdump")
+    out = subprocess.run([cuobjdump if os.path.exists(cuobjdump) else "cuobjdump", "-lelf", bf.SO_PATH], capture_output=True, text=True).stdout
     assert "sm_100a" in out
 
 
