@@ -1,5 +1,7 @@
 // tools/p2_bench.cu — Poseidon2 kernel-shape / pipe-balance experiments.  Each thread runs NPERM chained
 // permutations (like the leaf sponge: 32 per leaf); every variant must reproduce the baseline checksum.
+// The poseidon2.cuh switches apply to every row; build once per combination, e.g.
+//   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -DP2_SBOX_HI=1 -DP2_DIAG_SHIFT=2 -o p2_bench tools/p2_bench.cu
 #include <cuda_runtime.h>
 #include <cstdio>
 #include <cstring>
@@ -65,13 +67,15 @@ int main() {
     auto small = [](int v) { return v >= 0 ? kb::to_mont((uint32_t)v) : kb::neg(kb::to_mont((uint32_t)(-v))); };
     uint32_t dg[16] = {small(-2), small(1), small(2), frac(1, 1), small(3), small(4), frac(-1, 1), small(-3), small(-4), frac(1, 8), frac(1, 3), frac(1, 24), frac(-1, 8), frac(-1, 3), frac(-1, 4), frac(-1, 24)};
     memcpy(h.diag, dg, sizeof dg);
-    cudaMemcpyToSymbol(p2::c_p2, &h, sizeof h);
     ShoupC sc[16];
-    for (int i = 0; i < 16; i++) { uint32_t w = kb::from_mont(dg[i]); sc[i] = {w, (uint32_t)(((uint64_t)w << 32) / kb::P)}; }
+    for (int i = 0; i < 16; i++) { uint32_t w = kb::from_mont(dg[i]); sc[i] = {w, (uint32_t)(((uint64_t)w << 32) / kb::P)};
+                                   h.diag_w[i] = sc[i].w; h.diag_wp[i] = sc[i].wp; }
+    cudaMemcpyToSymbol(p2::c_p2, &h, sizeof h);
     cudaMemcpyToSymbol(c_diag_shoup, sc, sizeof sc);
     size_t n = 1 << 21;
     uint32_t* d; cudaMalloc(&d, n * 4);
     h_buf = (uint32_t*)malloc(n * 4);
+    printf("== P2_SBOX_HI=%d P2_DIAG_SHIFT=%d\n", P2_SBOX_HI, P2_DIAG_SHIFT);
     run<Base>("baseline (poseidon2.cuh rolled)", d, n);
     //            rc  m4 sum out isum iout lazy shoup
     run<Perm<Cfg<0, 0, 0, 0, 0, 0, false, 0>>>("variant, no forcing", d, n);

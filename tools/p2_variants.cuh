@@ -23,18 +23,11 @@ KB_D uint32_t subm(uint32_t a, uint32_t b, uint32_t big) {
     return umin_(d, d + P);
 }
 
+// lazy: the one-correction S-box of poseidon2.cuh (its P2_SBOX_HI form)
 template <bool LAZY>
 KB_D uint32_t sbox(uint32_t x) {
     if (!LAZY) return kb::mul(kb::mul(x, x), x);
-    uint64_t t = (uint64_t)x * x;
-    uint32_t m = (uint32_t)t * PINV;
-    uint32_t u = __umulhi(m, P);
-    int32_t x2 = (int32_t)((uint32_t)(t >> 32) - u);  // (-p, p), no correction
-    int64_t t2 = (int64_t)x2 * (int32_t)x;
-    int32_t m2 = (int32_t)((uint32_t)t2 * PINV);
-    int32_t u2 = __mulhi(m2, (int32_t)P);
-    uint32_t r = (uint32_t)((int32_t)(t2 >> 32) - u2);  // (-p, p) wrapped
-    return umin_(r, r + P);
+    return p2::sbox(x);
 }
 
 template <int RC_ALU, int M4_ALU, int SUM_ALU, int OUT_ALU, int ISUM_ALU, int IOUT_ALU, bool LAZY, int SHOUP /* 0 Montgomery, 1 Shoup, 2 shift-based 2^-k */>

@@ -17,6 +17,7 @@ __global__ void __launch_bounds__(256) k(uint32_t* out, uint32_t seed, uint32_t 
 #pragma unroll
     for (int i = 0; i < NCHAIN; i++) { a[i] = seed + threadIdx.x + i; w[i] = a[i]; }
     uint32_t y = seed * 3 + threadIdx.x, z = m ^ threadIdx.x;
+    const uint32_t rcs = z % P - P;  // a round constant stored as c - p
 #pragma unroll 1
     for (int it = 0; it < ITERS; it++) {
 #pragma unroll
@@ -64,6 +65,35 @@ __global__ void __launch_bounds__(256) k(uint32_t* out, uint32_t seed, uint32_t 
                 a[i] = a[i] * z + m;
                 uint32_t t = a[i] - P; a[i] = a[i] < t ? a[i] : t;
             }
+            if (KIND >= 14 && KIND <= 16) {                                                       // Poseidon2 S-box (poseidon2.cuh)
+                const int32_t x = (int32_t)(a[i] + rcs);  // [-p, p), as in the permutation
+                uint32_t r;
+                if (KIND == 16) {                         // 64-bit products, reduction fused into IMAD.HI's 64-bit addend
+                    uint32_t lo = (uint32_t)x * (uint32_t)x;
+                    int64_t t = (int64_t)(((uint64_t)(uint32_t)__mulhi(x, x) << 32) | lo);
+                    int32_t q = (int32_t)(lo * 0x81000001u);
+                    int32_t x2 = (int32_t)((t + (int64_t)q * -(int64_t)P) >> 32);
+                    uint32_t lo2 = (uint32_t)x2 * (uint32_t)x;
+                    int64_t t2 = (int64_t)(((uint64_t)(uint32_t)__mulhi(x2, x) << 32) | lo2);
+                    int32_t q2 = (int32_t)(lo2 * 0x81000001u);
+                    r = (uint32_t)(int32_t)((t2 + (int64_t)q2 * -(int64_t)P) >> 32);
+                } else if (KIND == 14) {                  // two 64-bit products
+                    int64_t t = (int64_t)x * x;
+                    uint32_t q = (uint32_t)t * 0x81000001u;
+                    int32_t x2 = (int32_t)((uint32_t)(t >> 32) - __umulhi(q, P));
+                    int64_t t2 = (int64_t)x2 * x;
+                    int32_t q2 = (int32_t)((uint32_t)t2 * 0x81000001u);
+                    r = (uint32_t)((int32_t)(t2 >> 32) - __mulhi(q2, (int32_t)P));
+                } else {                                  // low / high 32-bit products only
+                    uint32_t xp = (uint32_t)x * 0x81000001u;
+                    uint32_t q = (uint32_t)x * xp;
+                    int32_t x2 = __mulhi(x, x) - (int32_t)__umulhi(q, P);
+                    int32_t q2 = (int32_t)((uint32_t)x2 * xp);
+                    r = (uint32_t)(__mulhi(x2, x) - __mulhi(q2, (int32_t)P));
+                }
+                uint32_t r2 = r + P;
+                a[i] = r < r2 ? r : r2;
+            }
         }
     }
     uint32_t r = 0;
@@ -109,5 +139,8 @@ int main() {
     run<11>("IMAD + 2 VIADDMNMX", 3, sm);
     run<12>("IMAD + VIADDMNMX", 2, sm);
     run<13>("2 IMAD + VIADDMNMX", 3, sm);
+    run<14>("sbox (2 IMAD.WIDE+2 IMAD+2 IMAD.HI)", 10, sm);  // instr/step: SASS of the unrolled chain step (cuobjdump)
+    run<15>("sbox (3 IMAD+4 IMAD.HI)", 14.1, sm);  // 3.1 of them MOVs building IMAD.HI addend pairs
+    run<16>("sbox (2 IMAD.WIDE+2 IMAD+2 IMAD.HI fused)", 8, sm);
     return 0;
 }
