@@ -2,6 +2,8 @@
 // permutations (like the leaf sponge: 32 per leaf); every variant must reproduce the baseline checksum.
 // The poseidon2.cuh switches apply to every row; build once per combination, e.g.
 //   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -DP2_SBOX_HI=1 -DP2_DIAG_SHIFT=2 -o p2_bench tools/p2_bench.cu
+// Rows with the shift diagonal and no pinned internal-sum additions run poseidon2.cuh's internal layer, so a build with
+// -DP2_LAZY_LINEAR=0 against one without it compares the two internal-layer forms row by row.
 #include <cuda_runtime.h>
 #include <cstdio>
 #include <cstring>
@@ -75,7 +77,7 @@ int main() {
     size_t n = 1 << 21;
     uint32_t* d; cudaMalloc(&d, n * 4);
     h_buf = (uint32_t*)malloc(n * 4);
-    printf("== P2_SBOX_HI=%d P2_DIAG_SHIFT=%d\n", P2_SBOX_HI, P2_DIAG_SHIFT);
+    printf("== P2_SBOX_HI=%d P2_DIAG_SHIFT=%d P2_LAZY_LINEAR=%d\n", P2_SBOX_HI, P2_DIAG_SHIFT, P2_LAZY_LINEAR);
     run<Base>("baseline (poseidon2.cuh rolled)", d, n);
     //            rc  m4 sum out isum iout lazy shoup
     run<Perm<Cfg<0, 0, 0, 0, 0, 0, false, 0>>>("variant, no forcing", d, n);

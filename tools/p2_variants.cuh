@@ -138,7 +138,9 @@ struct Perm {
 #pragma unroll 1
                 for (int r = 0; r < 13; r++) {
                     s[0] = sbox<C::lazy>(addm<false>(s[0], p2::c_p2.internal[r], big));
-                    internal_linear(s);
+                    // shift diagonal, nothing pinned: the build's own layer (P2_LAZY_LINEAR picks its form)
+                    if constexpr (C::shoup == 2 && C::isum == 0) p2::internal_linear(s);
+                    else internal_linear(s);
                 }
             }
         }

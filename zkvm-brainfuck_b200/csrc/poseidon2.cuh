@@ -8,11 +8,13 @@
 // constants sit in constant memory in Montgomery form and are consumed as c[bank][imm] operands
 // (the permutation is fully unrolled).
 #pragma once
+#include <cstddef>
+
 #include "kb31.cuh"
 
 namespace p2 {
 
-struct Consts {
+struct alignas(16) Consts {  // 16-byte rows: permute() reads ext_s as uint4
     uint32_t ext[8][16];    // external rounds: 0..3 initial, 4..7 terminal (Montgomery form)
     uint32_t internal[16];  // 13 used
     uint32_t diag[16];      // internal diagonal V (Montgomery form), kept for reference/tests
@@ -21,6 +23,8 @@ struct Consts {
     uint32_t ext_s[8][16];  // ext - p and
     uint32_t internal_s[16];  // internal - p as wrapped 32-bit words: state + constant lands in [-p, p) with one plain add
 };
+
+static_assert(offsetof(Consts, ext_s) % 16 == 0, "ext_s rows are read as uint4");
 
 #if defined(__CUDACC__)
 // single translation unit (bfgpu.cu): the constant bank is defined here
@@ -161,18 +165,67 @@ KB_D void external_linear(uint32_t (&s)[16]) {
     }
 }
 
+// Lazy internal layer (P2_LAZY_LINEAR=1, default): the 15-word sum s[1] + ... + s[15] is one 64-bit carry chain and ONE
+// reduction instead of 14 modular additions, and the two halvings fold into the add of `sum`.  Every output stays in [0, p).
+//   - acc_wide: one mad.wide.u32 by 1 per word.  ptxas turns the chain into IADD3s with two carry-out predicates, each followed by
+//     an IADD3.X that adds both carries to the high word: 14 instructions for the 15 words, against 28 (IADD + VIADDMNMX per
+//     modular add).  Written as plain 64-bit additions, or as add.cc/addc pairs, it gets two-input IADD3s and 23 instructions.
+//   - reduce_wide: v < 15 p < 2^35.  With 2^31 = 2^24 - 1 (mod p), v = l + h 2^31 = l + h (2^24 - 1) where l = v mod 2^31 and
+//     h = v >> 31 <= 14 (one funnel shift, one AND, one IMAD); that is below 2^31 + 14 (2^24 - 1) < 2p, so one min-correction
+//     ends in [0, p).  4 instructions.
+//   - sum + x/2 with x/2 = (x >> 1) + (x & 1)(p + 1)/2: one IMAD puts the odd term on sum, one LEA.HI adds x >> 1, the total is
+//     below 2p: one correction, 4 instructions.  sum - x/2 is in (-p, p): one correction, 5 instructions.  Through kb::halve
+//     both cost 6 (a negation, a select mask and a separate modular add).  The mask is x & 0x80000001, which equals x & 1 for
+//     x < 2^31: with x & 1 ptxas knows the factor is 0 or 1 and turns the IMAD into a compare and a predicated move.
+// In `hashk::k_leaf_hash` the internal-round loop body drops from 127 to 114 SASS instructions (DESIGN 3.2).
+// tests/test_p2_linear.py restates every step with 32-bit semantics and asserts these bounds.
+#ifndef P2_LAZY_LINEAR
+#define P2_LAZY_LINEAR 1
+#endif
+KB_D uint64_t acc_wide(uint64_t acc, uint32_t x) {
+    asm("mad.wide.u32 %0, %1, 1, %0;" : "+l"(acc) : "r"(x));
+    return acc;
+}
+KB_D uint32_t reduce_wide(uint64_t v) {
+    const uint32_t lo = (uint32_t)v, r = (lo & 0x7fffffffu) + __funnelshift_l(lo, (uint32_t)(v >> 32), 1) * 0x00ffffffu;
+    return kb::umin_(r, r - kb::P);
+}
+KB_D uint32_t add_half(uint32_t sum, uint32_t x) {
+    const uint32_t r = (x & 0x80000001u) * ((kb::P + 1) / 2) + sum + (x >> 1);
+    return kb::umin_(r, r - kb::P);
+}
+KB_D uint32_t sub_half(uint32_t sum, uint32_t x) {
+    const uint32_t r = sum - (x & 0x80000001u) * ((kb::P + 1) / 2) - (x >> 1);
+    return kb::umin_(r, r + kb::P);
+}
+
 // 1 + Diag(V), V = [-2, 1, 2, 1/2, 3, 4, -1/2, -3, -4, 1/2^8, 1/8, 1/2^24, -1/2^8, -1/8, -1/16, -1/2^24]
 KB_D void internal_linear(uint32_t (&s)[16]) {
+#if P2_LAZY_LINEAR
+    uint64_t acc = 0;
+#pragma unroll
+    for (int i = 1; i < 16; i++) acc = acc_wide(acc, s[i]);
+    const uint32_t part = reduce_wide(acc);
+#else
     uint32_t part = add(add(add(s[1], s[2]), add(s[3], s[4])), add(add(s[5], s[6]), add(s[7], s[8])));
     part = add(part, add(add(add(s[9], s[10]), add(s[11], s[12])), add(add(s[13], s[14]), s[15])));
+#endif
     uint32_t sum = add(part, s[0]);
     s[0] = sub(part, s[0]);
     s[1] = add(s[1], sum);
     s[2] = add(dbl(s[2]), sum);
+#if P2_LAZY_LINEAR
+    s[3] = add_half(sum, s[3]);
+#else
     s[3] = add(kb::halve(s[3]), sum);
+#endif
     s[4] = add(add(dbl(s[4]), s[4]), sum);
     s[5] = add(dbl(dbl(s[5])), sum);
+#if P2_LAZY_LINEAR
+    s[6] = sub_half(sum, s[6]);
+#else
     s[6] = sub(sum, kb::halve(s[6]));
+#endif
     s[7] = sub(sum, add(dbl(s[7]), s[7]));
     s[8] = sub(sum, dbl(dbl(s[8])));
 #if P2_DIAG_SHIFT
@@ -213,8 +266,16 @@ KB_D void permute(uint32_t (&s)[16]) {
             const uint32_t* rc = c_p2.ext[half * 4 + r];
             const uint32_t* rcs = c_p2.ext_s[half * 4 + r];
             if (BARRIER) __syncthreads();
+            // the 16 signed round constants as 16-byte vectors: ptxas loads them with 8 LDCU.64 instead of 16 LDCU (the rolled
+            // loop indexes the constant bank, so each constant costs a uniform load; external-round body 292 -> 284 instructions)
 #pragma unroll
-            for (int i = 0; i < 16; i++) s[i] = sbox_rc(s[i], rc[i], rcs[i]);
+            for (int j = 0; j < 4; j++) {
+                const uint4 c = reinterpret_cast<const uint4*>(rcs)[j];
+                s[4 * j] = sbox_rc(s[4 * j], rc[4 * j], c.x);
+                s[4 * j + 1] = sbox_rc(s[4 * j + 1], rc[4 * j + 1], c.y);
+                s[4 * j + 2] = sbox_rc(s[4 * j + 2], rc[4 * j + 2], c.z);
+                s[4 * j + 3] = sbox_rc(s[4 * j + 3], rc[4 * j + 3], c.w);
+            }
             external_linear(s);
         }
         if (half == 0) {
