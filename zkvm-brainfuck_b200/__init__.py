@@ -507,8 +507,8 @@ class TwoAdicFriPcs:
         final_poly = take(4).astype(np.uint64)
         pow_witness = int(take(1)[0])
         nq = int(take(1)[0])
-        log_blowup = 1
-        log_max_height = ncommit + log_blowup
+        # FRI folds the tallest LDE down to 2^log_blowup entries, so the commit-phase layers follow from the heights alone
+        log_max_height = max(r for data, _ in rounds for r, _ in data.dims).bit_length() - 1
         queries = []
         for _ in range(nq):
             index = int(take(1)[0])
