@@ -114,6 +114,8 @@ enum {
     BFGPU_PHASE_QUOTIENT = 14,   /* quotient values                                                 */
     BFGPU_PHASE_EXCHANGE = 15,   /* multi-GPU commit: launches of the column->row exchange (they run on the copy stream) */
     BFGPU_PHASE_TRACEGEN = 16,   /* device-side trace generation from the execution record                          */
+    BFGPU_PHASE_DEBUG_ROWS = 17,    /* trace checker: constraint pass (bfgpu_machine_debug)                          */
+    BFGPU_PHASE_DEBUG_LOOKUPS = 18, /* trace checker: interaction pass (records, sort, reduction, gather)            */
     BFGPU_NUM_PHASES = 20
 };
 /* start (on != 0, clears the accumulators) or stop collecting per-phase timings */
@@ -277,6 +279,28 @@ int32_t bfgpu_machine_open(bfgpu_ctx* ctx, const bfgpu_pk* pk, const bfgpu_shard
 uint64_t bfgpu_shard_proof_size(const bfgpu_shard_proof* p);
 int32_t bfgpu_shard_proof_read(const bfgpu_shard_proof* p, uint32_t* out);
 void bfgpu_shard_proof_free(bfgpu_shard_proof* p);
+
+/* Trace checker: StarkMachine::debug_constraints (machine.rs:288-387, debug.rs:24-105, lookup/debug.rs:59-196) on the GPU.  Checks
+ * a committed shard without proving it: every constraint of every chip on every row (selectors exact, the next row of the last row
+ * is row 0), the LogUp cumulative sums, and the balance of every interaction (sends minus receives per (kind, values) over all
+ * chips).  Works on a COPY of `ch` (left unchanged): observes the main commitment and samples the LogUp (alpha, beta) exactly as
+ * bfgpu_machine_open does, so for a challenger in the state bfgpu_machine_open would receive the cumulative sums are the ones the
+ * proof carries; it then samples two more elements (gamma, delta) for the interaction fingerprints gamma + kind +
+ * sum_k delta^(k+1) value_k.  The reference's own sampling order inside debug_constraints cannot be checked offline; it does not
+ * affect the verdict, which depends on the challenges only through a fingerprint collision (probability ~ records^2 / p^4).
+ * The report is deterministic.  Flat u32 serialisation (caller representation for field elements):
+ *   n_chips; per chip in commit order: chip index (bfgpu_machine_chip_info), log_degree, cumulative_sum (4), n_failing,
+ *     per failing constraint (ascending index k in fold order: base constraints, one per LogUp batch column, then the LogUp
+ *     first-row, transition and last-row constraints): k, failing-row count, the min(count, max_rows) smallest failing natural rows;
+ *   total of the cumulative sums (4);
+ *   n_imbalanced; for the first min(n_imbalanced, max_keys) keys in (kind, canonical values) order: kind (LookupKind), n_values,
+ *     values (n_values), net multiplicity (sends - receives), n_chips with a nonzero net, then (chip index, net) per such chip. */
+typedef struct bfgpu_debug_report bfgpu_debug_report;
+int32_t bfgpu_machine_debug(bfgpu_ctx* ctx, const bfgpu_pk* pk, const bfgpu_shard* shard, const bfgpu_challenger* ch, uint32_t max_rows,
+                            uint32_t max_keys, bfgpu_debug_report** out);
+uint64_t bfgpu_debug_report_size(const bfgpu_debug_report* r);
+int32_t bfgpu_debug_report_read(const bfgpu_debug_report* r, uint32_t* out);
+void bfgpu_debug_report_free(bfgpu_debug_report* r);
 
 /* ---- plug point #2 (SURVEY.md §8b): the steps of CpuProver::open for an integration at the Plonky3 trait level ------------------------- */
 /* Pcs::get_evaluations_on_domain (prover.rs:365-373) as a device view: pointer and layout of the committed LDE (column-major,

@@ -142,6 +142,10 @@ ABI = {
     "bfgpu_shard_proof_size": (C.c_uint64, [C.c_void_p]),
     "bfgpu_shard_proof_read": (C.c_int32, [C.c_void_p, C.c_void_p]),
     "bfgpu_shard_proof_free": (None, [C.c_void_p]),
+    "bfgpu_machine_debug": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.POINTER(C.c_void_p)]),
+    "bfgpu_debug_report_size": (C.c_uint64, [C.c_void_p]),
+    "bfgpu_debug_report_read": (C.c_int32, [C.c_void_p, C.c_void_p]),
+    "bfgpu_debug_report_free": (None, [C.c_void_p]),
 }
 
 
@@ -230,7 +234,7 @@ class Context:
         self._pinned = []
 
     PHASES = ["h2d", "ingest", "intt", "scale", "ntt", "leaf_hash", "compress", "other", "open_eval", "open_reduce", "fri",
-              "pow", "query", "perm", "quotient", "exchange", "tracegen", "reserved17", "reserved18", "reserved19"]
+              "pow", "query", "perm", "quotient", "exchange", "tracegen", "debug_rows", "debug_lookups", "reserved19"]
 
     def profile_enable(self, on=True):
         self.check(lib().bfgpu_profile_enable(self._h, 1 if on else 0))
@@ -882,6 +886,31 @@ class CudaProver:
         finally:
             shard.free()
 
+    def debug_constraints(self, pk, shard, challenger, max_rows=5, max_keys=64):
+        """`StarkMachine::debug_constraints` (machine.rs:288-387) on the GPU: every constraint on every row and the balance of
+        every interaction of a committed shard (bfgpu_machine_debug).  `challenger` is left unchanged; in the state `open` would
+        receive (pk observed) the report's cumulative sums are the proof's.  Returns a DebugReport."""
+        h = C.c_void_p()
+        self.ctx.check(lib().bfgpu_machine_debug(self.ctx._h, pk._h, shard._h, challenger._h, int(max_rows), int(max_keys), C.byref(h)))
+        buf = np.zeros(lib().bfgpu_debug_report_size(h), np.uint32)
+        rc = lib().bfgpu_debug_report_read(h, _ptr(buf))
+        lib().bfgpu_debug_report_free(h)
+        self.ctx.check(rc)
+        return DebugReport(buf, [c[0] for c in self.chips], max_rows)
+
+    def debug_program(self, code, stdin=(), max_rows=5, max_keys=64):
+        """execute -> setup_record -> commit_record -> debug_constraints: checks the device trace generators on a program."""
+        rec = self.execute(code, stdin)
+        pk = self.setup_record(rec)
+        ch = Challenger(self.ctx)
+        lib().bfgpu_pk_observe_into(pk._h, ch._h)
+        shard = self.commit_record(rec)
+        try:
+            return self.debug_constraints(pk, shard, ch, max_rows, max_keys)
+        finally:
+            shard.free()
+            pk.free()
+
     def _parse(self, buf, pk, shard):
         info = {n: (mw, pw, ew, lo) for n, mw, pw, ew, lo in self.chips}
         com = dict(main=buf[0:8].copy(), permutation=buf[8:16].copy(), quotient=buf[16:24].copy())
@@ -926,6 +955,83 @@ class CudaProver:
             chips_out.append(dict(preprocessed=prep, main=lv(main_v[i], not lo), permutation=lv(perm_v[i], True),
                                   quotient=[quot_v[2 * i][0], quot_v[2 * i + 1][0]], cumulative_sum=csum, log_degree=log_degree))
         return dict(commitment=com, opened_values=chips_out, opening_proof=fri, chip_ordering={k: i for i, k in enumerate(names)})
+
+
+KIND_NAMES = {1: "Memory", 2: "Program", 3: "Alu", 4: "Jump", 5: "MemInstr", 6: "IO", 7: "Byte"}  # LookupKind (lookup.rs:19-41)
+_N_BASE = {}  # chip -> (base constraints, LogUp batch columns), from air/chips.py on first use
+
+
+def constraint_label(chip, k):
+    """Name of constraint k of a chip in fold order: "base k", "LogUp batch j", "LogUp first row" / "transition" / "last row"."""
+    if not _N_BASE:
+        from .air import chips as air_chips
+        _N_BASE.update({c.name: (len(c.constraints), c.perm_width - 1) for c in air_chips.machine_chips()})
+    n_base, n_batch = _N_BASE[chip]
+    if k < n_base:
+        return f"base {k}"
+    if k < n_base + n_batch:
+        return f"LogUp batch {k - n_base}"
+    return "LogUp " + ("first row", "transition", "last row")[k - n_base - n_batch]
+
+
+class DebugReport:
+    """Parsed bfgpu_machine_debug report (layout: include/bfgpu.h).
+      failures        [(chip, constraint index, label, failing-row count, first rows)] in (commit order, index) order
+      cumulative_sums {chip: (4,) words}, total: their sum (zero when the interactions balance)
+      imbalances      [(kind name, values tuple, net, {chip: net})] in (kind, values) order, at most max_keys of n_imbalanced
+      ok              no failing constraint, no imbalanced key, zero total"""
+
+    def __init__(self, words, chip_names, max_rows):
+        w = [int(x) for x in words]
+        pos = 0
+
+        def take(k=None):
+            nonlocal pos
+            pos += 1 if k is None else k
+            return w[pos - 1] if k is None else w[pos - k:pos]
+
+        self.words = np.asarray(words, np.uint32)
+        self.failures, self.cumulative_sums, self.log_degrees = [], {}, {}
+        for _ in range(take()):
+            chip = chip_names[take()]
+            self.log_degrees[chip] = take()
+            self.cumulative_sums[chip] = np.array(take(4), np.uint64)
+            for _ in range(take()):
+                k, count = take(), take()
+                self.failures.append((chip, k, constraint_label(chip, k), count, take(min(count, max_rows))))
+        self.total = np.array(take(4), np.uint64)
+        self.n_imbalanced = take()
+        self.imbalances = []
+        while pos < len(w):
+            kind, nv = take(), take()
+            values, net = tuple(take(nv)), take()
+            per_chip = {}
+            for _ in range(take()):
+                c = take()
+                per_chip[chip_names[c]] = take()
+            self.imbalances.append((KIND_NAMES[kind], values, net, per_chip))
+        self.ok = not self.failures and self.n_imbalanced == 0 and not self.total.any()
+
+    def __str__(self):
+        """The report in the reference's terms (debug.rs / lookup/debug.rs)."""
+        out = []
+        for chip, k, label, count, rows in self.failures:
+            more = f" (+{count - len(rows)} more)" if count > len(rows) else ""
+            out.append(f"constraint failed: chip {chip}, constraint {k} ({label}), {count} row(s): {', '.join(map(str, rows))}{more}")
+        out.append("constraints: ok" if not self.failures else f"constraints: {len(self.failures)} failing")
+        for kind, values, net, per_chip in self.imbalances:
+            chips = ", ".join(f"{c}: {_signed(v)}" for c, v in per_chip.items())
+            out.append(f"interaction imbalance: {kind} {list(values)}: net {_signed(net)} ({chips})")
+        if self.n_imbalanced > len(self.imbalances):
+            out.append(f"... {self.n_imbalanced - len(self.imbalances)} more imbalanced keys")
+        out.append("lookups: ok" if self.n_imbalanced == 0 and not self.total.any() else
+                   f"lookups: {self.n_imbalanced} imbalanced key(s), cumulative sums total {self.total.tolist()}")
+        return "\n".join(out)
+
+
+def _signed(v):
+    """A multiplicity mod p as the small signed integer it stands for (sends positive, receives negative)."""
+    return v - P if v > P // 2 else v
 
 
 # ---- sdk façade -----------------------------------------------------------------------------------------------------------

@@ -6,6 +6,9 @@ from the declarative AIR description in chips.py.  Straight-line code with commo
 all constants are emitted in Montgomery form.  Constraint k of a chip is folded as alpha^(N-1-k) * c_k, which
 equals the reference's Horner fold acc = acc * alpha + c_k.
 
+It also generates csrc/gen_air_debug.cuh, the row programs of the trace checker (per-constraint masks and raw interactions),
+and csrc/gen_air_ext.h / csrc/gen_layout.cuh (host verifier, trace generators).
+
 Run:  python -m zkvm-brainfuck_b200.air.codegen   (or importlib + main()); the output is committed.
 """
 import os
@@ -361,11 +364,126 @@ def generate_layout():
     return "\n".join(L) + "\n"
 
 
+# ---- trace checker (csrc/kernels_debug.cuh): constraint masks and raw interactions ------------------------------------------
+MASK_BITS = 64  # the constraint mask of one row is a uint64_t
+
+
+def gen_chip_debug(chip, index):
+    """`air_constraint_mask_<Chip>`: bit k set when constraint k (fold order: base constraints, one LogUp batch constraint per
+    batch column, then the first-row / transition / last-row LogUp constraints) is nonzero on the row, no alpha fold.
+    `air_lookups_<Chip>`: the row's sends and receives in `chip.lookups` order with their values and multiplicities."""
+    name = chip.name
+    n_base = len(chip.constraints)
+    W = chip.perm_width
+    total = n_base + (W - 1) + 3
+    assert total <= MASK_BITS, f"chip {name}: {total} constraints do not fit a {MASK_BITS}-bit row mask"
+    em = Emitter()
+    em.loaded = set()
+    names = _emit_dag(em, chip.constraints)
+    for n in topo_order(list(chip.constraints)):
+        if n.op == "var" and n.args[1] == 0:
+            em.loaded.add(f"{n.args[0][0]}0_{n.args[2]}")
+    em.emit("uint64_t m = 0;")
+    for k, c in enumerate(chip.constraints):
+        em.emit(f"m |= (uint64_t)({names[c._id]} != 0u) << {k};")
+    lookups = chip.lookups
+    for j in range(W - 1):
+        chunk = lookups[j * chip.batch_size:(j + 1) * chip.batch_size]
+        rl = []
+        for i, (lk, is_send) in enumerate(chunk):
+            r, m = _emit_rlc(em, lk, f"{j}_{i}")
+            rl.append((r, m, is_send))
+        em.emit(f"{{  // batch {j}: entry * prod(rlc) - sum_i m_i * prod_(j != i) rlc_j")
+        em.emit("    kb::Ext prod = " + rl[0][0] + ";")
+        for r, _, _ in rl[1:]:
+            em.emit(f"    prod = AIR_EXT_MUL(prod, {r});")
+        em.emit("    kb::Ext num = kb::ext_zero();")
+        for i, (r, m, is_send) in enumerate(rl):
+            others = [x[0] for k, x in enumerate(rl) if k != i]
+            if not others:
+                term = f"kb::ext_from_base({m})"
+            else:
+                o = others[0]
+                for x in others[1:]:
+                    o = f"AIR_EXT_MUL({o}, {x})"
+                term = f"kb::ext_scale({o}, {m})"
+            em.emit(f"    num = kb::ext_{'add' if is_send else 'sub'}(num, {term});")
+        em.emit(f"    m |= (uint64_t)ext_nonzero(kb::ext_sub(AIR_EXT_MUL(prod, ld.perm0({j})), num)) << {n_base + j};")
+        em.emit("}")
+    em.emit("{")
+    em.emit("    kb::Ext sum_local = kb::ext_zero(), sum_next = kb::ext_zero();")
+    for j in range(W - 1):
+        em.emit(f"    sum_local = kb::ext_add(sum_local, ld.perm0({j}));")
+        em.emit(f"    sum_next = kb::ext_add(sum_next, ld.perm1({j}));")
+    em.emit(f"    const kb::Ext phi_local = ld.perm0({W - 1}), phi_next = ld.perm1({W - 1});")
+    k0 = n_base + W - 1
+    em.emit(f"    m |= (uint64_t)ext_nonzero(kb::ext_scale(kb::ext_sub(phi_local, sum_local), sel.is_first)) << {k0};")
+    em.emit(f"    m |= (uint64_t)ext_nonzero(kb::ext_scale(kb::ext_sub(kb::ext_sub(phi_next, phi_local), sum_next), sel.is_trans)) << {k0 + 1};")
+    em.emit(f"    m |= (uint64_t)ext_nonzero(kb::ext_scale(kb::ext_sub(phi_local, ch.cumulative_sum), sel.is_last)) << {k0 + 2};")
+    em.emit("}")
+    em.emit("return m;")
+    out = [f"// ---- {name}: {n_base} base + {W - 1} LogUp batch + 3 LogUp boundary constraints, {len(lookups)} interactions"]
+    out.append(f"template <class L>\n__device__ __forceinline__ uint64_t air_constraint_mask_{name}(const L& ld, const Selectors& sel, const Challenges& ch) {{")
+    out += em.lines
+    out.append("}")
+    em = Emitter()
+    em.loaded = set()
+    for li, (lk, is_send) in enumerate(lookups):
+        em.emit(f"out[{li}].kind = {lk.kind};")
+        em.emit(f"out[{li}].is_send = {int(is_send)};")
+        em.emit(f"out[{li}].n_values = {len(lk.values)};")
+        for k, v in enumerate(lk.values):
+            val, _ = _affine_expr(em, v, f"{li}_{k}")
+            em.emit(f"out[{li}].v[{k}] = {val};")
+        m, _ = _affine_expr(em, lk.multiplicity, f"{li}_m")
+        em.emit(f"out[{li}].mult = {m};")
+    out.append(f"template <class L>\n__device__ __forceinline__ void air_lookups_{name}(const L& ld, LookupVals* out) {{")
+    out += em.lines
+    out.append("}")
+    return "\n".join(out), dict(name=name, index=index, n_lookups=len(lookups), max_values=max((len(lk.values) for lk, _ in lookups), default=0))
+
+
+def generate_debug():
+    chips = C.machine_chips()
+    parts, infos = [], []
+    for i, c in enumerate(chips):
+        code, info = gen_chip_debug(c, i)
+        parts.append(code)
+        infos.append(info)
+    hdr = ["// GENERATED by zkvm-brainfuck_b200/air/codegen.py from air/chips.py — do not edit.",
+           "// Row programs of the trace checker (csrc/kernels_debug.cuh): per-constraint nonzero masks in fold order and the raw",
+           "// interactions of a row.  Included by kernels_debug.cuh after kernels_air.cuh (Selectors, Challenges, AIR_EXT_MUL).",
+           "#pragma once", "namespace air {",
+           f"constexpr int MAX_LOOKUPS = {max(i['n_lookups'] for i in infos)};",
+           f"constexpr int MAX_LOOKUP_VALUES = {max(i['max_values'] for i in infos)};",
+           "struct LookupVals {  // one send or receive of a row: LookupKind, direction, values and multiplicity (Montgomery words)",
+           "    uint32_t kind, is_send, n_values, mult;",
+           "    uint32_t v[MAX_LOOKUP_VALUES];",
+           "};",
+           "__device__ __forceinline__ bool ext_nonzero(const kb::Ext& e) { return (e.c[0] | e.c[1] | e.c[2] | e.c[3]) != 0u; }",
+           "__host__ __device__ constexpr int num_lookups(int chip) {",
+           "    return " + " : ".join(f"chip == {i['index']} ? {i['n_lookups']}" for i in infos) + " : 0;",
+           "}"]
+    disp = ["template <class L>\n__device__ __forceinline__ uint64_t air_constraint_mask(int chip, const L& ld, const Selectors& sel, const Challenges& ch) {",
+            "    switch (chip) {"]
+    for inf in infos:
+        disp.append(f"        case {inf['index']}: return air_constraint_mask_{inf['name']}(ld, sel, ch);")
+    disp.append("    }\n    return 0;\n}")
+    disp.append("template <class L>\n__device__ __forceinline__ void air_lookups(int chip, const L& ld, LookupVals* out) {")
+    disp.append("    switch (chip) {")
+    for inf in infos:
+        disp.append(f"        case {inf['index']}: air_lookups_{inf['name']}(ld, out); break;")
+    disp.append("    }\n}")
+    return "\n".join(hdr) + "\n\n" + "\n\n".join(parts) + "\n\n" + "\n".join(disp) + "\n}  // namespace air\n"
+
+
 def main():
     with open(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "csrc", "gen_layout.cuh"), "w") as f:
         f.write(generate_layout())
     with open(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "csrc", "gen_air_ext.h"), "w") as f:
         f.write(generate_ext())
+    with open(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "csrc", "gen_air_debug.cuh"), "w") as f:
+        f.write(generate_debug())
     out = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "csrc", "gen_air.cuh")
     src = generate()
     with open(out, "w") as f:

@@ -4,6 +4,8 @@
     python bfprove.py prove    prog.bf [--stdin 17] --out proof          # needs a GPU; writes proof.bfproof, proof.bin, proof.vk.json
     python bfprove.py verify   proof.bfproof --vk proof.vk.json           # no GPU: native host verifier, exit status 0 = accepted
     python bfprove.py size     proof.bfproof --vk proof.vk.json           # the reference's `proofSize` (bincode bytes)
+    python bfprove.py check    prog.bf [--stdin 17]                     # needs a GPU: every constraint and interaction of the
+                                                                        # generated traces (debug_constraints); exit status 0 = clean
 
 `prove` prints the reference's summary line (crates/core/machine/src/utils/prove.rs:50-56): cycles, e2e ms, kHz, proofSize.
 File formats: *.bfproof = the flat little-endian u32 serialisation of include/bfgpu.h (bfgpu_machine_open), canonical words;
@@ -45,6 +47,12 @@ def main(argv=None):
     p.add_argument("--stdin", default="")
     p.add_argument("--out", default="proof")
     p.add_argument("--device", type=int, default=0)
+    k = sub.add_parser("check")
+    k.add_argument("program")
+    k.add_argument("--stdin", default="")
+    k.add_argument("--device", type=int, default=0)
+    k.add_argument("--max-rows", type=int, default=5)
+    k.add_argument("--max-keys", type=int, default=64)
     for name in ("verify", "size"):
         v = sub.add_parser(name)
         v.add_argument("proof")
@@ -75,6 +83,15 @@ def main(argv=None):
         print(f"summary: cycles={cycles}, e2e={ms:.0f}, khz={cycles / ms:.2f}, proofSize={_human(len(blob))}")
         del ctx
         return 0
+    if args.cmd == "check":
+        from . import Context, CudaProver
+        ctx = Context(args.device)
+        try:
+            report = CudaProver(ctx).debug_program(open(args.program).read(), _stdin_bytes(args.stdin), args.max_rows, args.max_keys)
+        finally:
+            ctx.close()
+        print(report)
+        return 0 if report.ok else 1
     vk = json.load(open(args.vk))
     words = np.fromfile(args.proof, dtype="<u4")
     fri = vk.get("fri", dict(log_blowup=1, num_queries=84, pow_bits=16))

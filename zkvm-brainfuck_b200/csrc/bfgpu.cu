@@ -3011,6 +3011,280 @@ static int32_t quotient_values_impl(bfgpu_ctx* ctx, const char* chip, const bfgp
 }
 
 // =====================================================================================================
+// trace checker: StarkMachine::debug_constraints (machine.rs:288-387, debug.rs:24-105, lookup/debug.rs:59-196)
+// =====================================================================================================
+#include "kernels_debug.cuh"
+
+struct bfgpu_debug_report {
+    std::vector<uint32_t> flat;
+};
+
+// Memory: the LogUp traces (16 B x perm_w per row), one 8-byte mask per row, and for the interaction pass R records
+// (R <= sum of rows x lookups: 2^26 + 2^23.5 for 2^22 Cpu rows) held as two key/value buffers for the sort (2 x 24 B), the
+// per-fingerprint aggregates (36 B) and the imbalanced-group indices (4 B): 88 B per record plus CUB's scratch, about 7 GB at
+// 2^22 Cpu rows.  Everything is scratch of this call; only the flat report survives it.
+static int32_t machine_debug_impl(bfgpu_ctx* ctx, const bfgpu_pk* pk, const bfgpu_shard* sd, const bfgpu_challenger* chh, uint32_t max_rows,
+                                  uint32_t max_keys, bfgpu_debug_report** out);
+extern "C" int32_t bfgpu_machine_debug(bfgpu_ctx* ctx, const bfgpu_pk* pk, const bfgpu_shard* sd, const bfgpu_challenger* chh, uint32_t max_rows,
+                                       uint32_t max_keys, bfgpu_debug_report** out) {
+    AllocScope scope(ctx);  // blocks taken by a failing call go back to the cache (see AllocScope)
+    return scope.ok(machine_debug_impl(ctx, pk, sd, chh, max_rows, max_keys, out));
+}
+static int32_t machine_debug_impl(bfgpu_ctx* ctx, const bfgpu_pk* pk, const bfgpu_shard* sd, const bfgpu_challenger* chh, uint32_t max_rows,
+                                  uint32_t max_keys, bfgpu_debug_report** out) {
+    if (!ctx || !pk || !sd || !chh || !out) return fail(ctx, BFGPU_ERR_INVALID, "null argument");
+    *out = nullptr;
+    const size_t nchips = sd->names.size();
+    if (nchips > 16) return fail(ctx, BFGPU_ERR_INVALID, "the checker handles at most 16 traces per shard");
+    std::vector<int> pk_idx(nchips, -1);
+    for (size_t i = 0; i < nchips; i++)
+        for (size_t k = 0; k < pk->names.size(); k++)
+            if (pk->names[k] == sd->names[i]) pk_idx[i] = (int)k;
+    for (size_t i = 0; i < nchips; i++) {
+        const air::ChipInfo& ci = air::CHIPS[sd->chip[i]];
+        if (ci.prep_w && (pk_idx[i] < 0 || pk->traces[pk_idx[i]].rows != sd->traces[i].rows))
+            return fail(ctx, BFGPU_ERR_INVALID, "chip %s: preprocessed trace missing or of a different height", ci.name);
+        if (sd->traces[i].rows > (1ull << 24)) return fail(ctx, BFGPU_ERR_INVALID, "chip %s: more than 2^24 rows", ci.name);
+    }
+    // ---- transcript on a copy: main commitment, LogUp (alpha, beta) as machine_open, then the fingerprint challenges ----------
+    bfgpu_challenger ch = box(chh)->ch;
+    ch.observe_slice(sd->commit, 8);
+    air::Challenges chal;
+    chal.alpha = ch.sample_ext();
+    const kb::Ext beta = ch.sample_ext();
+    chal.beta_pow[0] = kb::ext_one();
+    for (int k = 1; k < 8; k++) chal.beta_pow[k] = kb::ext_mul(chal.beta_pow[k - 1], beta);
+    chal.cumulative_sum = kb::ext_zero();
+    dbg::Fingerprint fp;
+    fp.gamma = ch.sample_ext();
+    const kb::Ext delta = ch.sample_ext();
+    fp.delta_pow[0] = kb::ext_one();
+    for (int k = 1; k <= air::MAX_LOOKUP_VALUES; k++) fp.delta_pow[k] = kb::ext_mul(fp.delta_pow[k - 1], delta);
+
+    Scratch sc(ctx);
+    // ---- LogUp traces and cumulative sums (the prover's own kernels) ----------------------------------------------------------
+    std::vector<DMat> perm(nchips);
+    std::vector<kb::Ext> csum(nchips);
+    uint32_t* d_csums = nullptr;
+    TRY(sc.alloc((void**)&d_csums, nchips * 16));
+    TRY(perm_traces(ctx, pk, pk_idx, sd->chip, sd->traces, chal, &perm, d_csums));
+    for (DMat& m : perm) sc.bufs.push_back(m.d);
+    CU(cudaMemcpyAsync(csum.data(), d_csums, nchips * 16, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));  // the last-row constraint of each chip compares with its cumulative sum
+
+    // ---- constraint pass ----------------------------------------------------------------------------------------------------
+    std::vector<uint64_t*> masks(nchips, nullptr);
+    std::vector<uint32_t*> bcounts(nchips, nullptr);
+    std::vector<uint32_t> totals(nchips * 64);
+    {
+        Phase ph(ctx, BFGPU_PHASE_DEBUG_ROWS);
+        uint32_t* d_totals = nullptr;
+        TRY(sc.alloc((void**)&d_totals, nchips * 64 * 4));
+        CU(cudaMemsetAsync(d_totals, 0, nchips * 64 * 4, ctx->stream));
+        for (size_t i = 0; i < nchips; i++) {
+            const uint64_t n = sd->traces[i].rows;
+            const unsigned log_n = ilog2(n);
+            const uint64_t nb = (n + dbg::MASK_BLOCK - 1) / dbg::MASK_BLOCK;
+            TRY(sc.alloc((void**)&masks[i], n * 8));
+            TRY(sc.alloc((void**)&bcounts[i], nb * 64 * 4));
+            air::Challenges c2 = chal;
+            c2.cumulative_sum = csum[i];
+            const uint32_t* prep = pk_idx[i] >= 0 ? pk->traces[pk_idx[i]].d : nullptr;
+#define BF_DBG_CASE(C) \
+    case C: dbg::k_debug_rows<C><<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>(sd->traces[i].d, prep, perm[i].d, log_n, c2, masks[i]); break;
+            switch (sd->chip[i]) {
+                BF_DBG_CASE(0) BF_DBG_CASE(1) BF_DBG_CASE(2) BF_DBG_CASE(3) BF_DBG_CASE(4) BF_DBG_CASE(5) BF_DBG_CASE(6) BF_DBG_CASE(7)
+            }
+#undef BF_DBG_CASE
+            LAUNCHED(ctx);
+            CU(cudaGetLastError());
+            dbg::k_mask_counts<<<(unsigned)nb, 256, 0, ctx->stream>>>(masks[i], n, bcounts[i], d_totals + 64 * i);
+            LAUNCHED(ctx);
+            CU(cudaGetLastError());
+        }
+        CU(cudaMemcpyAsync(totals.data(), d_totals, nchips * 64 * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    }
+
+    // ---- interaction pass ---------------------------------------------------------------------------------------------------
+    uint64_t rmax = 0;
+    for (size_t i = 0; i < nchips; i++) rmax += sd->traces[i].rows * (uint64_t)air::num_lookups(sd->chip[i]);
+    if (rmax >= (1ull << 31)) return fail(ctx, BFGPU_ERR_INVALID, "too many interactions for the checker (%llu)", (unsigned long long)rmax);
+    uint64_t n_bad = 0;
+    std::vector<uint32_t> gathered;
+    {
+        Phase ph(ctx, BFGPU_PHASE_DEBUG_LOOKUPS);
+        dbg::FpKey *keys_a = nullptr, *keys_b = nullptr;
+        uint64_t *vals_a = nullptr, *vals_b = nullptr;
+        unsigned long long* d_count = nullptr;
+        TRY(sc.alloc((void**)&d_count, 16));
+        TRY(sc.alloc((void**)&keys_a, std::max<uint64_t>(rmax, 1) * sizeof(dbg::FpKey)));
+        TRY(sc.alloc((void**)&vals_a, std::max<uint64_t>(rmax, 1) * 8));
+        TRY(sc.alloc((void**)&keys_b, std::max<uint64_t>(rmax, 1) * sizeof(dbg::FpKey)));
+        TRY(sc.alloc((void**)&vals_b, std::max<uint64_t>(rmax, 1) * 8));
+        CU(cudaMemsetAsync(d_count, 0, 16, ctx->stream));
+        for (size_t i = 0; i < nchips; i++) {
+            const uint64_t n = sd->traces[i].rows;
+            const unsigned log_n = ilog2(n);
+            const uint32_t* prep = pk_idx[i] >= 0 ? pk->traces[pk_idx[i]].d : nullptr;
+#define BF_REC_CASE(C)                                                                                                                          \
+    case C:                                                                                                                                     \
+        dbg::k_debug_records<C><<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>(sd->traces[i].d, prep, log_n, (uint32_t)i, fp, keys_a, vals_a, \
+                                                                                      d_count);                                                 \
+        break;
+            switch (sd->chip[i]) {
+                BF_REC_CASE(0) BF_REC_CASE(1) BF_REC_CASE(2) BF_REC_CASE(3) BF_REC_CASE(4) BF_REC_CASE(5) BF_REC_CASE(6) BF_REC_CASE(7)
+            }
+#undef BF_REC_CASE
+            LAUNCHED(ctx);
+            CU(cudaGetLastError());
+        }
+        unsigned long long nrec = 0;
+        CU(cudaMemcpyAsync(&nrec, d_count, 8, cudaMemcpyDeviceToHost, ctx->stream));
+        CU(cudaStreamSynchronize(ctx->stream));
+        if (nrec) {
+            const int R = (int)nrec;
+            size_t sort_bytes = 0, red_bytes = 0;
+            CU(cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, keys_a, keys_b, vals_a, vals_b, R, dbg::FpDecomposer{}, ctx->stream));
+            int* d_chip_of_pos = nullptr;
+            int* d_ngroups = nullptr;
+            dbg::Group* groups = nullptr;
+            uint32_t* bad = nullptr;
+            std::vector<int> chip_of_pos(16, 0);
+            for (size_t i = 0; i < nchips; i++) chip_of_pos[i] = sd->chip[i];
+            TRY(sc.alloc((void**)&d_chip_of_pos, 16 * sizeof(int)));
+            TRY(upload_small(ctx, d_chip_of_pos, chip_of_pos.data(), 16 * sizeof(int)));
+            const auto grp_in = thrust::make_transform_iterator(vals_b, dbg::RecordToGroup{d_chip_of_pos});
+            CU(cub::DeviceReduce::ReduceByKey(nullptr, red_bytes, keys_b, keys_a, grp_in, (dbg::Group*)nullptr, d_ngroups, dbg::GroupSum{}, R, ctx->stream));
+            void* temp = nullptr;
+            TRY(sc.alloc(&temp, std::max(sort_bytes, red_bytes)));
+            TRY(sc.alloc((void**)&groups, (size_t)R * sizeof(dbg::Group)));
+            TRY(sc.alloc((void**)&bad, (size_t)R * 4));
+            TRY(sc.alloc((void**)&d_ngroups, 16));
+            CU(cub::DeviceRadixSort::SortPairs(temp, sort_bytes, keys_a, keys_b, vals_a, vals_b, R, dbg::FpDecomposer{}, ctx->stream));
+            LAUNCHED(ctx);
+            CU(cub::DeviceReduce::ReduceByKey(temp, red_bytes, keys_b, keys_a, grp_in, groups, d_ngroups, dbg::GroupSum{}, R, ctx->stream));
+            LAUNCHED(ctx);
+            CU(cudaMemsetAsync(d_count, 0, 8, ctx->stream));
+            dbg::k_imbalanced<<<(unsigned)((R + 255) / 256), 256, 0, ctx->stream>>>(groups, d_ngroups, bad, d_count);
+            LAUNCHED(ctx);
+            CU(cudaGetLastError());
+            unsigned long long nb = 0;
+            CU(cudaMemcpyAsync(&nb, d_count, 8, cudaMemcpyDeviceToHost, ctx->stream));
+            CU(cudaStreamSynchronize(ctx->stream));
+            n_bad = nb;
+            if (n_bad) {
+                dbg::TraceRef tr{};
+                for (size_t i = 0; i < nchips; i++) {
+                    tr.main[i] = sd->traces[i].d;
+                    tr.prep[i] = pk_idx[i] >= 0 ? pk->traces[pk_idx[i]].d : nullptr;
+                    tr.log_n[i] = ilog2(sd->traces[i].rows);
+                    tr.chip[i] = sd->chip[i];
+                }
+                uint32_t* d_out = nullptr;
+                TRY(sc.alloc((void**)&d_out, n_bad * dbg::GATHER_WORDS * 4));
+                dbg::k_gather_values<<<(unsigned)((n_bad + 63) / 64), 64, 0, ctx->stream>>>(tr, groups, bad, n_bad, d_out);
+                LAUNCHED(ctx);
+                CU(cudaGetLastError());
+                gathered.resize(n_bad * dbg::GATHER_WORDS);
+                CU(cudaMemcpyAsync(gathered.data(), d_out, gathered.size() * 4, cudaMemcpyDeviceToHost, ctx->stream));
+            }
+        }
+    }
+    CU(cudaStreamSynchronize(ctx->stream));
+
+    // ---- failing rows: exact counts from the totals, the first max_rows rows from the count blocks that hold them ------------------
+    auto* rep = new bfgpu_debug_report();
+    std::unique_ptr<bfgpu_debug_report> rep_guard(rep);
+    auto& flat = rep->flat;
+    flat.push_back((uint32_t)nchips);
+    kb::Ext total = kb::ext_zero();
+    for (size_t i = 0; i < nchips; i++) {
+        const uint64_t n = sd->traces[i].rows;
+        const int nk = air::CHIPS[sd->chip[i]].n_constraints;
+        flat.push_back((uint32_t)sd->chip[i]);
+        flat.push_back(ilog2(n));
+        for (int k = 0; k < 4; k++) flat.push_back(out_word(ctx, csum[i].c[k]));
+        total = kb::ext_add(total, csum[i]);
+        const uint32_t* tot = &totals[64 * i];
+        int nfail = 0;
+        for (int k = 0; k < nk; k++) nfail += tot[k] != 0;
+        flat.push_back((uint32_t)nfail);
+        if (!nfail) continue;
+        const uint64_t nb = (n + dbg::MASK_BLOCK - 1) / dbg::MASK_BLOCK;
+        std::vector<uint32_t> bc(nb * 64);
+        CU(cudaMemcpy(bc.data(), bcounts[i], bc.size() * 4, cudaMemcpyDeviceToHost));
+        std::vector<char> need(nb, 0);
+        for (int k = 0; k < nk; k++) {
+            uint64_t want = std::min<uint64_t>(tot[k], max_rows);
+            for (uint64_t b = 0; b < nb && want; b++)
+                if (bc[b * 64 + k]) {
+                    need[b] = 1;
+                    want -= std::min<uint64_t>(want, bc[b * 64 + k]);
+                }
+        }
+        std::vector<std::vector<uint32_t>> rows(nk);
+        std::vector<uint64_t> blk(dbg::MASK_BLOCK);
+        for (uint64_t b = 0; b < nb; b++) {
+            if (!need[b]) continue;
+            const uint64_t r0 = b * dbg::MASK_BLOCK, cnt = std::min<uint64_t>(dbg::MASK_BLOCK, n - r0);
+            CU(cudaMemcpy(blk.data(), masks[i] + r0, cnt * 8, cudaMemcpyDeviceToHost));
+            for (uint64_t r = 0; r < cnt; r++)
+                for (uint64_t m = blk[r]; m; m &= m - 1) {
+                    const int k = __builtin_ctzll(m);
+                    if (rows[k].size() < max_rows) rows[k].push_back((uint32_t)(r0 + r));
+                }
+        }
+        for (int k = 0; k < nk; k++) {
+            if (!tot[k]) continue;
+            flat.push_back((uint32_t)k);
+            flat.push_back(tot[k]);
+            flat.insert(flat.end(), rows[k].begin(), rows[k].end());
+        }
+    }
+    for (int k = 0; k < 4; k++) flat.push_back(out_word(ctx, total.c[k]));
+
+    // ---- imbalanced keys, ordered by (kind, canonical values) ------------------------------------------------------------------
+    std::vector<uint64_t> order(n_bad);
+    std::vector<std::vector<uint32_t>> sort_key(n_bad);
+    for (uint64_t b = 0; b < n_bad; b++) {
+        const uint32_t* g = &gathered[b * dbg::GATHER_WORDS];
+        order[b] = b;
+        sort_key[b].push_back(g[0]);
+        for (uint32_t v = 0; v < g[1]; v++) sort_key[b].push_back(kb::from_mont(g[2 + v]));
+    }
+    std::sort(order.begin(), order.end(), [&](uint64_t a, uint64_t b) { return sort_key[a] < sort_key[b]; });
+    flat.push_back((uint32_t)n_bad);
+    for (uint64_t j = 0; j < std::min<uint64_t>(n_bad, max_keys); j++) {
+        const uint32_t* g = &gathered[order[j] * dbg::GATHER_WORDS];
+        const uint32_t* net = g + 2 + air::MAX_LOOKUP_VALUES;
+        flat.push_back(g[0]);
+        flat.push_back(g[1]);
+        for (uint32_t v = 0; v < g[1]; v++) flat.push_back(out_word(ctx, g[2 + v]));
+        uint32_t s = 0, nc = 0;
+        for (int c = 0; c < air::NUM_CHIPS; c++) {
+            s = kb::add(s, net[c]);
+            nc += net[c] != 0;
+        }
+        flat.push_back(out_word(ctx, s));
+        flat.push_back(nc);
+        for (int c = 0; c < air::NUM_CHIPS; c++)
+            if (net[c]) {
+                flat.push_back((uint32_t)c);
+                flat.push_back(out_word(ctx, net[c]));
+            }
+    }
+    *out = rep_guard.release();
+    return BFGPU_OK;
+}
+extern "C" uint64_t bfgpu_debug_report_size(const bfgpu_debug_report* r) { return r ? r->flat.size() : 0; }
+extern "C" int32_t bfgpu_debug_report_read(const bfgpu_debug_report* r, uint32_t* out) {
+    if (!r || !out) return BFGPU_ERR_INVALID;
+    memcpy(out, r->flat.data(), r->flat.size() * 4);
+    return BFGPU_OK;
+}
+extern "C" void bfgpu_debug_report_free(bfgpu_debug_report* r) { delete r; }
+
+// =====================================================================================================
 // one commitment over several GPUs
 // =====================================================================================================
 #include "dist_commit.cuh"
