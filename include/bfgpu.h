@@ -116,6 +116,7 @@ enum {
     BFGPU_PHASE_TRACEGEN = 16,   /* device-side trace generation from the execution record                          */
     BFGPU_PHASE_DEBUG_ROWS = 17,    /* trace checker: constraint pass (bfgpu_machine_debug)                          */
     BFGPU_PHASE_DEBUG_LOOKUPS = 18, /* trace checker: interaction pass (records, sort, reduction, gather)            */
+    BFGPU_PHASE_VERIFY = 19,        /* batch verifier: plan upload, query checks, result bits back (bfgpu_verify_batch) */
     BFGPU_NUM_PHASES = 20
 };
 /* start (on != 0, clears the accumulators) or stop collecting per-phase timings */
@@ -392,6 +393,27 @@ int32_t bfgpu_verify_shard_ex(const uint32_t vk_commit[8], const char* const* pr
 int32_t bfgpu_verify_core_proof(const uint32_t vk_commit[8], const char* const* prep_names, const uint32_t* prep_log_heights, int32_t n_prep,
                                 const uint32_t* proof, uint64_t n_words, int repr, uint32_t log_blowup, uint32_t num_queries,
                                 uint32_t pow_bits, const uint32_t* options, int32_t n_options, char* err, uint64_t err_len);
+
+/* ---- batch verifier on the device ---------------------------------------------------------------------------- */
+/* One proof of a batch: its verifying key (as for bfgpu_verify_shard) and its serialised words. */
+typedef struct {
+    const uint32_t* vk_commit;
+    const char* const* prep_names;
+    const uint32_t* prep_log_heights;
+    int32_t n_prep;
+    const uint32_t* proof;
+    uint64_t n_words;
+} bfgpu_verify_item;
+/* `BfProver::verify` (crates/prover/src/verify.rs:10-36) when core is 1, else `Verifier::verify_shard` (crates/stark/src/verifier.rs:27-329),
+ * for n_items proofs in one call.  The host parses and shape-checks each proof, replays its transcript, checks the proof of work and
+ * evaluates the constraints at zeta; the Merkle openings of every query (input and commit-phase rounds), the reduced openings and the
+ * fold chain of every proof run on the device in one pass.  status[i] and the string at errs + i * err_len (truncated to err_len bytes,
+ * errs may be NULL when err_len is 0) are exactly what bfgpu_verify_core_proof (core = 1) or bfgpu_verify_shard_ex (core = 0) return for
+ * item i under the same repr, FRI parameters and options.  The return value reports only bad arguments or device failures
+ * (bfgpu_last_error); n_items = 0 does nothing.  Runs on the context's stream and synchronises it. */
+int32_t bfgpu_verify_batch(bfgpu_ctx* ctx, const bfgpu_verify_item* items, int32_t n_items, int repr, uint32_t log_blowup, uint32_t num_queries,
+                           uint32_t pow_bits, const uint32_t* options, int32_t n_options, int32_t core, int32_t* status, char* errs,
+                           uint64_t err_len);
 
 /* Canonical proof serialiser (SURVEY.md §8f item 2): the bytes `bincode::serialize(&MachineProof { shard_proof })` writes for this proof
  * (crates/stark/src/types.rs:32-73,116-119; bincode 1.x defaults) — what the reference's `proofSize` counts

@@ -98,6 +98,8 @@ ABI = {
                               _u32p, C.c_int32, C.c_char_p, C.c_uint64]),
     "bfgpu_verify_core_proof": (C.c_int32, [_u32p, C.POINTER(C.c_char_p), _u32p, C.c_int32, _u32p, C.c_uint64, C.c_int, C.c_uint32, C.c_uint32, C.c_uint32,
                                 _u32p, C.c_int32, C.c_char_p, C.c_uint64]),
+    "bfgpu_verify_batch": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int, C.c_uint32, C.c_uint32, C.c_uint32, _u32p, C.c_int32, C.c_int32,
+                                       C.POINTER(C.c_int32), C.c_char_p, C.c_uint64]),
     "bfgpu_shard_proof_to_bincode": (C.c_int32, [C.POINTER(C.c_char_p), _u32p, C.c_int32, _u32p, C.c_uint64, C.c_int, C.c_uint32, C.c_int, C.c_void_p,
                                                   C.c_uint64, _u64p, C.c_char_p, C.c_uint64]),
     "bfgpu_dist_commit_begin": (C.c_int32, [C.c_void_p, C.c_uint32, C.c_uint32, _u64p, _u32p, C.c_int32, C.POINTER(C.c_void_p)]),
@@ -147,6 +149,11 @@ ABI = {
     "bfgpu_debug_report_read": (C.c_int32, [C.c_void_p, C.c_void_p]),
     "bfgpu_debug_report_free": (None, [C.c_void_p]),
 }
+
+
+class VerifyItem(C.Structure):
+    _fields_ = [("vk_commit", _u32p), ("prep_names", C.POINTER(C.c_char_p)), ("prep_log_heights", _u32p), ("n_prep", C.c_int32), ("proof", _u32p),
+                ("n_words", C.c_uint64)]
 
 
 class OpenRound(C.Structure):
@@ -234,7 +241,7 @@ class Context:
         self._pinned = []
 
     PHASES = ["h2d", "ingest", "intt", "scale", "ntt", "leaf_hash", "compress", "other", "open_eval", "open_reduce", "fri",
-              "pow", "query", "perm", "quotient", "exchange", "tracegen", "debug_rows", "debug_lookups", "reserved19"]
+              "pow", "query", "perm", "quotient", "exchange", "tracegen", "debug_rows", "debug_lookups", "verify"]
 
     def profile_enable(self, on=True):
         self.check(lib().bfgpu_profile_enable(self._h, 1 if on else 0))
@@ -641,6 +648,28 @@ def verify_core_proof(vk_commit, prep_names, prep_heights, proof_words, log_blow
     at most 22 (CpuLogDegreeTooLarge: n), then `StarkMachine::verify` -> `verify_shard`, whose errors read "InvalidShardProof: ...".
     Returns None when accepted.  Needs no GPU."""
     return verify_shard(vk_commit, prep_names, prep_heights, proof_words, log_blowup, num_queries, pow_bits, repr, options, core=True)
+
+
+def verify_batch(ctx, items, log_blowup=1, num_queries=84, pow_bits=16, repr=REPR_CANONICAL, options=None, core=True):
+    """Verify many serialised proofs in one device call (bfgpu_verify_batch).  items: list of (vk_commit, prep_names, prep_heights,
+    proof_words).  Returns one entry per item: None when accepted, else exactly the string `verify_core_proof` (core=True) or
+    `verify_shard` (core=False) returns for it."""
+    keep = []
+    arr = (VerifyItem * max(len(items), 1))()
+    for i, (com, names, heights, words) in enumerate(items):
+        com, words = _u32(com), _u32(words)
+        cn = (C.c_char_p * max(len(names), 1))(*[n.encode() for n in names])
+        logs = _u32([int(h).bit_length() - 1 for h in heights])
+        keep += [com, words, cn, logs]
+        arr[i] = VerifyItem(com.ctypes.data_as(_u32p), cn, logs.ctypes.data_as(_u32p), len(names), words.ctypes.data_as(_u32p), words.size)
+    opt = _u32([1, 0, 0])  # defaults of bfgpu_set_transcript_option
+    for k, v in (options or {}).items():
+        opt[Context.OPTIONS[k]] = int(v)
+    status = (C.c_int32 * max(len(items), 1))()
+    errs = C.create_string_buffer(256 * max(len(items), 1))
+    ctx.check(lib().bfgpu_verify_batch(ctx._h, C.byref(arr), len(items), repr, log_blowup, num_queries, pow_bits, opt.ctypes.data_as(_u32p), 3, int(core),
+                                       status, errs, 256))
+    return [None if status[i] == 0 else (errs.raw[256 * i:256 * (i + 1)].split(b"\0")[0].decode() or f"error {status[i]}") for i in range(len(items))]
 
 
 def proof_to_bincode(prep_names, prep_heights, proof_words, log_blowup=1, repr=REPR_CANONICAL, field_repr=1):

@@ -3,6 +3,9 @@
     python bfprove.py execute  prog.bf [--stdin 17]
     python bfprove.py prove    prog.bf [--stdin 17] --out proof          # needs a GPU; writes proof.bfproof, proof.bin, proof.vk.json
     python bfprove.py verify   proof.bfproof --vk proof.vk.json           # no GPU: native host verifier, exit status 0 = accepted
+    python bfprove.py verify   a.bfproof b.bfproof --vk a.vk.json [--vk b.vk.json] [--device 0]
+                                                                        # one line per proof, exit status 0 = all accepted; --device:
+                                                                        # all of them in one GPU call (bfgpu_verify_batch)
     python bfprove.py size     proof.bfproof --vk proof.vk.json           # the reference's `proofSize` (bincode bytes)
     python bfprove.py check    prog.bf [--stdin 17]                     # needs a GPU: every constraint and interaction of the
                                                                         # generated traces (debug_constraints); exit status 0 = clean
@@ -36,7 +39,7 @@ def _human(nbytes):
 
 
 def main(argv=None):
-    from . import ProverClient, Record, proof_to_bincode, verify_core_proof
+    from . import ProverClient, Record, proof_to_bincode, verify_batch, verify_core_proof
     ap = argparse.ArgumentParser(prog="bfprove", description=__doc__, formatter_class=argparse.RawDescriptionHelpFormatter)
     sub = ap.add_subparsers(dest="cmd", required=True)
     e = sub.add_parser("execute")
@@ -53,10 +56,13 @@ def main(argv=None):
     k.add_argument("--device", type=int, default=0)
     k.add_argument("--max-rows", type=int, default=5)
     k.add_argument("--max-keys", type=int, default=64)
-    for name in ("verify", "size"):
-        v = sub.add_parser(name)
-        v.add_argument("proof")
-        v.add_argument("--vk", required=True)
+    v = sub.add_parser("size")
+    v.add_argument("proof")
+    v.add_argument("--vk", required=True)
+    v = sub.add_parser("verify")
+    v.add_argument("proof", nargs="+")
+    v.add_argument("--vk", required=True, action="append", help="once for all proofs, or once per proof")
+    v.add_argument("--device", type=int, default=None, help="verify all proofs in one call on this GPU")
     args = ap.parse_args(argv)
 
     if args.cmd == "execute":
@@ -92,19 +98,35 @@ def main(argv=None):
             ctx.close()
         print(report)
         return 0 if report.ok else 1
-    vk = json.load(open(args.vk))
-    words = np.fromfile(args.proof, dtype="<u4")
-    fri = vk.get("fri", dict(log_blowup=1, num_queries=84, pow_bits=16))
     if args.cmd == "size":
+        vk = json.load(open(args.vk))
+        words = np.fromfile(args.proof, dtype="<u4")
+        fri = vk.get("fri", dict(log_blowup=1, num_queries=84, pow_bits=16))
         blob = proof_to_bincode(vk["names"], vk["heights"], words, fri["log_blowup"])
         print(f"proofSize={_human(len(blob))} ({len(blob)} bytes; {words.size} field/shape words in the flat form)")
         return 0
-    err = verify_core_proof(np.array(vk["commit"], np.uint32), vk["names"], vk["heights"], words, fri["log_blowup"], fri["num_queries"], fri["pow_bits"])
-    if err is None:
-        print("accepted")
-        return 0
-    print(f"rejected: {err}")
-    return 1
+    if len(args.vk) not in (1, len(args.proof)):
+        ap.error("--vk must be given once, or once per proof")
+    vks = [json.load(open(f)) for f in args.vk]
+    vks = vks * len(args.proof) if len(vks) == 1 else vks
+    frl = [vk.get("fri", dict(log_blowup=1, num_queries=84, pow_bits=16)) for vk in vks]
+    proofs = [np.fromfile(f, dtype="<u4") for f in args.proof]
+    if args.device is None:
+        errs = [verify_core_proof(np.array(vk["commit"], np.uint32), vk["names"], vk["heights"], words, fri["log_blowup"], fri["num_queries"],
+                                  fri["pow_bits"]) for vk, fri, words in zip(vks, frl, proofs)]
+    else:
+        if any(fri != frl[0] for fri in frl):
+            ap.error("--device verifies in one call: every verifying key must name the same FRI parameters")
+        from . import Context
+        ctx = Context(args.device)
+        try:
+            errs = verify_batch(ctx, [(np.array(vk["commit"], np.uint32), vk["names"], vk["heights"], words) for vk, words in zip(vks, proofs)],
+                                frl[0]["log_blowup"], frl[0]["num_queries"], frl[0]["pow_bits"])
+        finally:
+            ctx.close()
+    for err in errs:
+        print("accepted" if err is None else f"rejected: {err}")
+    return 0 if all(err is None for err in errs) else 1
 
 
 if __name__ == "__main__":

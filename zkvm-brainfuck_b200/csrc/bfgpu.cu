@@ -120,6 +120,9 @@ struct bfgpu_ctx {
     unsigned dist_fri_gather_log = 20;  // dist_prove.cuh: global FRI length below which the sharded prover gathers ($BFGPU_DIST_FRI_GATHER_LOG)
     // test hook (bfgpu_debug_fail_alloc): the n-th dalloc from now fails with BFGPU_ERR_OOM
     int64_t fail_alloc_in = -1;
+    // page-locked staging buffer of bfgpu_verify_batch (plan records and query words up, result bits down), grown on demand
+    uint8_t* vstage = nullptr;
+    size_t vstage_size = 0;
 };
 
 struct bfgpu_tree {
@@ -414,6 +417,7 @@ extern "C" void bfgpu_ctx_destroy(bfgpu_ctx* ctx) {
     if (ctx->d_tw) cudaFree(ctx->d_tw);
     if (ctx->d_inv256) cudaFree(ctx->d_inv256);
     if (ctx->ring) cudaFreeHost(ctx->ring);
+    if (ctx->vstage) cudaFreeHost(ctx->vstage);
     {
         std::lock_guard<std::mutex> g(g_ctx_mutex);
         g_live_ctx.erase(ctx);
@@ -3304,3 +3308,206 @@ extern "C" void bfgpu_debug_report_free(bfgpu_debug_report* r) { delete r; }
 // native verifier (host only)
 // =====================================================================================================
 #include "verifier.h"
+
+// =====================================================================================================
+// batch verifier: host stage per proof (verifier::prepare), query checks on the device (kernels_verify.cuh)
+// =====================================================================================================
+#include <atomic>
+#include <thread>
+
+#include "kernels_verify.cuh"
+
+namespace vfy {
+// host stage of one batch item: the verdict the host decides by itself (outer: before the shard verifier, the `BfProver::verify`
+// checks; inner: the shard verifier's), or the plan the device completes
+struct Item {
+    std::string outer, inner, cons;
+    bool decided = false;
+    verifier::Plan pl;
+    uint32_t bits = 0;  // first result bit (device items)
+    bool device = false;
+};
+// verifier::walk over the device's result bits
+struct BitChecks {
+    const uint32_t* bits;
+    uint32_t base, nc;
+    bool get(uint32_t q, uint32_t c) const {
+        const uint32_t b = base + q * nc + c;
+        return bits && ((bits[b >> 5] >> (b & 31)) & 1);
+    }
+    bool input(uint32_t q, int r) const { return get(q, (uint32_t)r); }
+    bool commit(uint32_t q, uint32_t k) const { return get(q, 4 + k); }
+    bool final_ok(uint32_t q) const { return get(q, nc - 1); }
+};
+template <class F>
+static void parallel_for(int n, F fn) {
+    const int nt = std::max(1, std::min<int>({n, (int)std::thread::hardware_concurrency(), 16}));
+    std::atomic<int> next{0};
+    auto work = [&] {
+        for (int i; (i = next.fetch_add(1)) < n;) fn(i);
+    };
+    std::vector<std::thread> th;
+    for (int t = 1; t < nt; t++) th.emplace_back(work);
+    work();
+    for (auto& t : th) t.join();
+}
+static size_t align16(size_t b) { return (b + 15) & ~(size_t)15; }
+}  // namespace vfy
+
+extern "C" int32_t bfgpu_verify_batch(bfgpu_ctx* ctx, const bfgpu_verify_item* items, int32_t n_items, int repr, uint32_t log_blowup,
+                                      uint32_t num_queries, uint32_t pow_bits, const uint32_t* options, int32_t n_options, int32_t core,
+                                      int32_t* status, char* errs, uint64_t err_len) {
+    if (!ctx) return BFGPU_ERR_INVALID;
+    if (n_items < 0 || (n_items && (!items || !status || (err_len && !errs)))) return fail(ctx, BFGPU_ERR_INVALID, "bfgpu_verify_batch: null argument");
+    if (n_items == 0) return BFGPU_OK;
+    AllocScope scope(ctx);
+    uint32_t opt[BFGPU_NUM_OPTS];
+    verifier::parse_options(options, n_options, opt);
+    const bool monty = repr == BFGPU_REPR_MONTY;
+    std::vector<vfy::Item> it(n_items);
+    // host stage: the checks of bfgpu_verify_core_proof / bfgpu_verify_shard_ex up to the queries, the query plan, the constraints at zeta
+    vfy::parallel_for(n_items, [&](int i) {
+        auto& x = it[i];
+        const auto& a = items[i];
+        x.decided = true;
+        if (core) {
+            if (!a.vk_commit || !a.proof) {
+                x.outer = "null argument";
+                return;
+            }
+            if (!(x.outer = verifier::core_precheck(a.proof, a.n_words)).empty()) return;
+        }
+        if (!a.vk_commit || !a.proof || a.n_prep < 0 || (a.n_prep && (!a.prep_names || !a.prep_log_heights))) {
+            x.inner = "null argument";
+            return;
+        }
+        std::vector<std::pair<int, unsigned>> prep;
+        if (!(x.inner = verifier::parse_prep(a.prep_names, a.prep_log_heights, a.n_prep, prep)).empty()) return;
+        if (!(x.inner = verifier::prepare(a.vk_commit, prep, a.proof, a.n_words, monty, log_blowup, num_queries, pow_bits, opt, x.pl)).empty()) return;
+        x.cons = verifier::constraints(x.pl);
+        x.decided = false;
+        x.device = x.pl.tall_round < 0;  // else the walk stops at query 0 before any check
+    });
+    // ---- plan -> device records
+    std::vector<vfy::VProof> P;
+    std::vector<vfy::VMat> M;
+    std::vector<uint32_t> aux;
+    std::vector<int> owner;
+    uint64_t n_words = 0, n_leaf = 0;
+    uint32_t n_bits = 0, n_fold = 0, n_merkle = 0;
+    for (int i = 0; i < n_items; i++) {
+        auto& x = it[i];
+        if (x.decided || !x.device) continue;
+        const auto& pl = x.pl;
+        vfy::VProof v{};
+        v.words = n_words;
+        v.leaf = n_leaf;
+        v.bits = x.bits = n_bits;
+        v.task = n_fold;
+        v.mtask = n_merkle;
+        v.nq = pl.nq_eff;
+        v.stride = (uint32_t)pl.stride;
+        v.monty = monty;
+        v.log_max = pl.log_max;
+        v.n_commit = pl.n_commit;
+        v.rollin = pl.opt[BFGPU_OPT_FRI_ROLLIN];
+        for (int r = 0; r < 4; r++) {
+            v.round_off[r] = pl.round_off[r];
+            v.sib_off[r] = pl.sib_off[r];
+            v.round_lbm[r] = pl.round_lbm[r];
+        }
+        v.aux = (uint32_t)aux.size();
+        aux.insert(aux.end(), pl.index.begin(), pl.index.end());
+        aux.insert(aux.end(), pl.cp_off.begin(), pl.cp_off.end());
+        for (auto& b : pl.betas) aux.insert(aux.end(), b.c, b.c + 4);
+        for (auto& c : pl.fri_commits) aux.insert(aux.end(), c.begin(), c.end());
+        for (auto& r : pl.rounds) aux.insert(aux.end(), r.commit, r.commit + 8);
+        aux.insert(aux.end(), pl.fri_alpha.c, pl.fri_alpha.c + 4);
+        aux.insert(aux.end(), pl.final_poly.c, pl.final_poly.c + 4);
+        for (int r = 0; r < 4; r++) {
+            v.mat[r] = (uint32_t)M.size();
+            for (auto& m : pl.rounds[r].mats) {
+                M.push_back(vfy::VMat{m.log_n + pl.log_blowup, m.width, (uint32_t)m.points.size(), (uint32_t)aux.size()});
+                for (auto& z : m.points) aux.insert(aux.end(), z.c, z.c + 4);
+                for (auto& vals : m.values)
+                    for (auto& e : vals) aux.insert(aux.end(), e.c, e.c + 4);
+            }
+        }
+        v.mat[4] = (uint32_t)M.size();
+        P.push_back(v);
+        owner.push_back(i);
+        n_words += (uint64_t)pl.nq_eff * pl.stride;
+        n_leaf += (uint64_t)pl.nq_eff * pl.n_commit;
+        n_bits += pl.nq_eff * (5 + pl.n_commit);
+        n_fold += pl.nq_eff;
+        n_merkle += pl.nq_eff * (4 + pl.n_commit);
+    }
+    std::vector<uint32_t> bits((n_bits + 31) / 32, 0);
+    if (!P.empty()) {
+        // one page-locked staging buffer: [proofs | matrices | aux words | query words], then the result bits coming back
+        const size_t oP = 0, oM = vfy::align16(P.size() * sizeof(vfy::VProof)), oA = oM + vfy::align16(M.size() * sizeof(vfy::VMat)),
+                     oW = oA + vfy::align16(aux.size() * 4), in_bytes = oW + vfy::align16(n_words * 4), out_bytes = bits.size() * 4;
+        if (ctx->vstage_size < in_bytes + out_bytes) {
+            if (ctx->vstage) {
+                CU(cudaStreamSynchronize(ctx->stream));
+                cudaFreeHost(ctx->vstage);
+                ctx->vstage = nullptr;
+                ctx->vstage_size = 0;
+            }
+            const size_t want = std::max<size_t>(in_bytes + out_bytes, 1 << 20) * 5 / 4;
+            CU(cudaHostAlloc((void**)&ctx->vstage, want, cudaHostAllocDefault));
+            ctx->vstage_size = want;
+        }
+        uint8_t* st = ctx->vstage;
+        memcpy(st + oP, P.data(), P.size() * sizeof(vfy::VProof));
+        memcpy(st + oM, M.data(), M.size() * sizeof(vfy::VMat));
+        memcpy(st + oA, aux.data(), aux.size() * 4);
+        vfy::parallel_for((int)P.size(), [&](int j) {
+            const auto& pl = it[owner[j]].pl;
+            const auto& a = items[owner[j]];
+            uint32_t* dst = (uint32_t*)(st + oW) + P[j].words;
+            const uint64_t need = (uint64_t)pl.nq_eff * pl.stride, have = std::min<uint64_t>(need, a.n_words - pl.q_base);
+            memcpy(dst, a.proof + pl.q_base, have * 4);
+            memset(dst + have, 0, (need - have) * 4);  // past a truncation: stages the walk never reads
+        });
+        Phase ph(ctx, BFGPU_PHASE_VERIFY);
+        Scratch s(ctx);
+        uint8_t* d_in;
+        uint32_t* d_work;
+        TRY(s.alloc((void**)&d_in, in_bytes));
+        TRY(s.alloc((void**)&d_work, (n_leaf * 8 + bits.size()) * 4));
+        uint32_t* d_bits = d_work + n_leaf * 8;
+        CU(cudaMemcpyAsync(d_in, st, in_bytes, cudaMemcpyHostToDevice, ctx->stream));
+        CU(cudaMemsetAsync(d_bits, 0, bits.size() * 4, ctx->stream));
+        const auto* dP = (const vfy::VProof*)(d_in + oP);
+        const auto* dM = (const vfy::VMat*)(d_in + oM);
+        const auto* dA = (const uint32_t*)(d_in + oA);
+        const auto* dW = (const uint32_t*)(d_in + oW);
+        vfy::k_verify_fold<<<(n_fold + 127) / 128, 128, 0, ctx->stream>>>(dP, (int)P.size(), dM, dA, dW, n_fold, d_work, d_bits);
+        LAUNCHED(ctx);
+        vfy::k_verify_merkle<<<(n_merkle + 127) / 128, 128, 0, ctx->stream>>>(dP, (int)P.size(), dM, dA, dW, n_merkle, d_work, d_bits);
+        LAUNCHED(ctx);
+        CU(cudaGetLastError());
+        uint32_t* back = (uint32_t*)(st + in_bytes);
+        CU(cudaMemcpyAsync(back, d_bits, out_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+        CU(cudaStreamSynchronize(ctx->stream));
+        memcpy(bits.data(), back, out_bytes);
+    }
+    // ---- the first failing event of every proof, in the host verifier's order
+    for (int i = 0; i < n_items; i++) {
+        auto& x = it[i];
+        std::string e = x.outer;
+        if (e.empty()) {
+            std::string in = x.inner;
+            if (!x.decided) {
+                vfy::BitChecks bc{x.device ? bits.data() : nullptr, x.bits, 5 + x.pl.n_commit};
+                in = verifier::walk(x.pl, bc);
+                if (in.empty()) in = x.cons;
+            }
+            e = core ? verifier::core_wrap(in) : in;
+        }
+        status[i] = e.empty() ? BFGPU_OK : BFGPU_ERR_INVALID;
+        verifier::say(errs ? errs + (size_t)i * err_len : nullptr, err_len, e);
+    }
+    return scope.ok();
+}

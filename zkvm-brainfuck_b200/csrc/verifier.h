@@ -10,6 +10,7 @@
 #pragma once
 #include <cstdarg>
 #include <map>
+#include <set>
 #include <string>
 #include <vector>
 
@@ -145,25 +146,64 @@ static std::string fmt(const char* f, ...) {
     return buf;
 }
 
-// returns "" when the proof is accepted, else the reference's error name (+ detail)
-static std::string verify(const uint32_t vk_commit_in[8], const std::vector<std::pair<int, unsigned>>& prep /* (chip index, log height), pk order */,
-                          const uint32_t* words, uint64_t n_words, bool monty, unsigned log_blowup, unsigned num_queries, unsigned pow_bits,
-                          const uint32_t opt[BFGPU_NUM_OPTS]) {
+struct ChipOpen {
+    int chip;
+    unsigned log_degree;
+    Ext csum;
+};
+
+// The query phase of one proof, laid out before any of it is checked.  Where a word sits in the proof depends only on the shape
+// words read before the queries, never on whether a check passed, so the host stage (`prepare`) can place every query's words,
+// replay the whole transcript and find where the reader would stop; an executor then computes every check of the plan (host:
+// HostChecks; device: kernels_verify.cuh) and `walk` reports the first failing event in the order `verify` meets them.
+struct Plan {
+    bool monty;
+    unsigned log_blowup, log_max, n_commit;
+    uint32_t nq;      // queries of the proof (= num_queries)
+    uint32_t nq_eff;  // queries up to and including the one the reader stops in
+    uint32_t opt[BFGPU_NUM_OPTS];
+    std::vector<std::pair<int, unsigned>> prep;
+    Round rounds[4];
+    std::vector<ChipOpen> chips;
+    Ext perm_ch[2], alpha, zeta, fri_alpha, final_poly;
+    std::vector<std::array<uint32_t, 8>> fri_commits;
+    std::vector<Ext> betas;
+    std::vector<uint32_t> index;  // sampled query indices (nq_eff)
+    uint64_t q_base, stride;      // word position of query 0 and words per query
+    // per input round: first opened-row word, first sibling word (both relative to the query's index word), log2 of the tallest LDE
+    uint32_t round_off[4], sib_off[4], round_lbm[4];
+    std::vector<uint32_t> cp_off;  // per FRI round: first word of the commit-phase opening (sibling value, then path)
+    int tall_round = -1;           // first round with a matrix taller than the FRI domain
+    bool rollin_bad = false;       // a reduced opening at a height the fold chain never rolls in
+    // stage 0: the index word; 1..4: input round stage-1; 5 + k: commit-phase round k.  stop_q == nq: the reader reads every query
+    uint32_t stop_q, stop_stage = 0;
+    bool index_word_differs = false, trailing = false;
+};
+
+// Everything up to the queries: shapes, opened values, transcript, proof of work, and the query plan.  Returns "" when the
+// proof reaches its queries, else the error `verify` returns before them.
+static std::string prepare(const uint32_t vk_commit_in[8], const std::vector<std::pair<int, unsigned>>& prep /* (chip index, log height), pk order */,
+                           const uint32_t* words, uint64_t n_words, bool monty, unsigned log_blowup, unsigned num_queries, unsigned pow_bits,
+                           const uint32_t opt[BFGPU_NUM_OPTS], Plan& pl) {
     Reader rd{words, n_words, 0, monty};
+    pl.monty = monty;
+    pl.log_blowup = log_blowup;
+    pl.prep = prep;
+    memcpy(pl.opt, opt, sizeof pl.opt);
     uint32_t vk_commit[8];
     for (int i = 0; i < 8; i++) {
         if (vk_commit_in[i] >= kb::P) return "InvalidProofShape: non-canonical verifying key";
         vk_commit[i] = monty ? vk_commit_in[i] : kb::to_mont(vk_commit_in[i]);
     }
-    Round rounds[4];
+    Round* rounds = pl.rounds;
     memcpy(rounds[0].commit, vk_commit, 32);
     rd.digest(rounds[1].commit);
     rd.digest(rounds[2].commit);
     rd.digest(rounds[3].commit);
     const uint32_t n = rd.raw();
     if (!rd.ok || n == 0 || n > (uint32_t)air::NUM_CHIPS) return "ChipOpeningLengthMismatch";
-    struct ChipOpen { int chip; unsigned log_degree; Ext csum; };
-    std::vector<ChipOpen> chips(n);
+    auto& chips = pl.chips;
+    chips.resize(n);
     std::map<int, size_t> where;
     for (auto& c : chips) {
         c.chip = (int)rd.raw();
@@ -179,12 +219,13 @@ static std::string verify(const uint32_t vk_commit_in[8], const std::vector<std:
     ch.observe_slice(vk_commit, 8);
     for (int i = 0; i < 7; i++) ch.observe(0);
     ch.observe_slice(rounds[1].commit, 8);
-    Ext perm_ch[2] = {ch.sample_ext(), ch.sample_ext()};
+    pl.perm_ch[0] = ch.sample_ext();
+    pl.perm_ch[1] = ch.sample_ext();
     ch.observe_slice(rounds[2].commit, 8);
     for (auto& c : chips) ch.observe_ext(c.csum);
-    const Ext alpha = ch.sample_ext();
+    pl.alpha = ch.sample_ext();
     ch.observe_slice(rounds[3].commit, 8);
-    const Ext zeta = ch.sample_ext();
+    const Ext zeta = pl.zeta = ch.sample_ext();
     auto next_point = [&](unsigned log_n) { return kb::ext_scale(zeta, kb::two_adic_generator(log_n)); };
     // ---- opening rounds: shapes, then the opened values in serialisation order ---------------------------------------------
     for (auto& pr : prep) {
@@ -201,13 +242,13 @@ static std::string verify(const uint32_t vk_commit_in[8], const std::vector<std:
         rounds[2].mats.push_back(OpenedMat{c.log_degree, 4u * (uint32_t)info.perm_w, {zeta, next_point(c.log_degree)}, {}});
         for (int d = 0; d < (1 << info.log_quotient_degree); d++) rounds[3].mats.push_back(OpenedMat{c.log_degree, 4, {zeta}, {}});
     }
-    for (auto& r : rounds) {
-        if (r.mats.empty()) return "InvalidProofShape: commitment round without matrices";
-        for (auto& m : r.mats)
+    for (int r = 0; r < 4; r++) {
+        if (rounds[r].mats.empty()) return "InvalidProofShape: commitment round without matrices";
+        for (auto& m : rounds[r].mats)
             if (m.log_n > (unsigned)kb::TWO_ADICITY - log_blowup) return "InvalidProofShape";
     }
-    for (auto& r : rounds)
-        for (auto& m : r.mats)
+    for (int r = 0; r < 4; r++)
+        for (auto& m : rounds[r].mats)
             for (size_t t = 0; t < m.points.size(); t++) {
                 std::vector<Ext> v(m.width);
                 for (auto& e : v) e = rd.ext();
@@ -215,122 +256,220 @@ static std::string verify(const uint32_t vk_commit_in[8], const std::vector<std:
             }
     if (!rd.ok) return "InvalidProofShape: truncated opened values";
     // ---- TwoAdicFriPcs::verify ------------------------------------------------------------------------------------------------
-    for (auto& r : rounds)
-        for (auto& m : r.mats)
+    for (int r = 0; r < 4; r++)
+        for (auto& m : rounds[r].mats)
             for (auto& v : m.values)
                 for (auto& e : v)
                     if (opt[BFGPU_OPT_OBSERVE_OPENED_VALUES]) ch.observe_ext(e);
-    const Ext fri_alpha = ch.sample_ext();
-    const uint32_t n_commit = rd.raw();
+    pl.fri_alpha = ch.sample_ext();
+    const uint32_t n_commit = pl.n_commit = rd.raw();
     if (!rd.ok || n_commit == 0 || n_commit > (unsigned)kb::TWO_ADICITY - log_blowup) return "InvalidProofShape";
     for (auto& c : chips)  // every committed LDE must fit under the first FRI layer
         if (c.log_degree > n_commit) return "InvalidProofShape: chip taller than the FRI domain";
-    std::vector<std::array<uint32_t, 8>> fri_commits(n_commit);
-    std::vector<Ext> betas(n_commit);
+    pl.fri_commits.resize(n_commit);
+    pl.betas.resize(n_commit);
     for (uint32_t k = 0; k < n_commit; k++) {
-        rd.digest(fri_commits[k].data());
-        ch.observe_slice(fri_commits[k].data(), 8);
-        betas[k] = ch.sample_ext();
+        rd.digest(pl.fri_commits[k].data());
+        ch.observe_slice(pl.fri_commits[k].data(), 8);
+        pl.betas[k] = ch.sample_ext();
     }
-    const Ext final_poly = rd.ext();
-    ch.observe_ext(final_poly);
+    pl.final_poly = rd.ext();
+    ch.observe_ext(pl.final_poly);
     const uint32_t pow_witness = rd.raw();  // canonical in the serialisation
-    const uint32_t nq = rd.raw();
+    const uint32_t nq = pl.nq = rd.raw();
     if (!rd.ok || nq != num_queries) return "InvalidProofShape: query count";
     // every error of pcs.verify reaches the caller wrapped (verifier.rs: `.map_err(VerificationError::InvalidopeningArgument)`)
     if (pow_witness >= kb::P || !ch.check_witness(pow_bits, kb::to_mont(pow_witness))) return "InvalidOpeningArgument:InvalidPowWitness";
-    const unsigned log_max = n_commit + log_blowup;
-    const uint32_t gen = kb::to_mont(kb::GEN);
-    bool index_word_differs = false;
-    for (uint32_t qi = 0; qi < nq; qi++) {
-        const uint32_t index = ch.sample_bits(log_max);
+    // ---- query layout: index word, per input round the opened rows then the Merkle path, per FRI round the sibling value then the path
+    const unsigned log_max = pl.log_max = n_commit + log_blowup;
+    uint64_t off = 1;
+    std::set<unsigned, std::greater<unsigned>> heights;
+    for (int r = 0; r < 4; r++) {
+        unsigned lbm = 0;
+        uint64_t w = 0;
+        for (auto& m : rounds[r].mats) {
+            lbm = std::max(lbm, m.log_n + log_blowup);
+            w += m.width;
+            heights.insert(m.log_n + log_blowup);
+        }
+        if (lbm > log_max && pl.tall_round < 0) pl.tall_round = r;
+        pl.round_off[r] = (uint32_t)off;
+        pl.sib_off[r] = (uint32_t)(off + w);
+        pl.round_lbm[r] = lbm;
+        off += w + 8ull * lbm;
+    }
+    pl.cp_off.resize(n_commit);
+    for (uint32_t k = 0; k < n_commit; k++) {
+        pl.cp_off[k] = (uint32_t)off;
+        off += 4 + 8ull * (log_max - 1 - k);
+    }
+    pl.stride = off;
+    pl.q_base = rd.pos;
+    // the fold chain rolls in the reduced opening of height log_max - k before folding round k; any other height is left over
+    auto hit = heights.begin();
+    for (uint32_t k = 0; k < n_commit; k++)
+        if (hit != heights.end() && *hit == log_max - k) ++hit;
+    pl.rollin_bad = hit != heights.end();
+    // the reader's stop: the first word past the end, or a field word (every word of a query but its index) outside [0, p)
+    pl.stop_q = nq;
+    for (uint64_t q = 0; q < nq && pl.stop_q == nq; q++) {
+        const uint64_t base = pl.q_base + q * pl.stride;
+        for (uint64_t o = 0; o < pl.stride; o++) {
+            if (base + o >= n_words || (o && words[base + o] >= kb::P)) {
+                pl.stop_q = (uint32_t)q;
+                if (o >= pl.round_off[0]) pl.stop_stage = 1;
+                for (int r = 1; r < 4; r++)
+                    if (o >= pl.round_off[r]) pl.stop_stage = 1 + r;
+                for (uint32_t k = 0; k < n_commit; k++)
+                    if (o >= pl.cp_off[k]) pl.stop_stage = 5 + k;
+                break;
+            }
+        }
+    }
+    pl.nq_eff = pl.stop_q < nq ? pl.stop_q + 1 : nq;
+    pl.index.resize(pl.nq_eff);
+    for (uint32_t q = 0; q < pl.nq_eff; q++) {
+        pl.index[q] = ch.sample_bits(log_max);
         // The serialisation carries the index for the reader's convenience; the reference's QueryProof does not, its verifier uses the
         // sampled one.  So a transcript that went wrong fails where the reference fails (the Merkle openings no longer fit the sampled
         // index: InputMmcsError); a proof that verifies but carries another index word is a second encoding of the same proof and is
         // refused at the end.
-        if (rd.raw() != index) index_word_differs = true;
-        if (!rd.ok) return "InvalidProofShape: truncated query";
-        // reduced openings per height (fri/two_adic_pcs.rs verify: open_input)
-        std::map<unsigned, Ext, std::greater<unsigned>> ro;
-        std::map<unsigned, Ext> apow;
-        for (auto& r : rounds) {
-            std::vector<uint64_t> heights;
-            std::vector<std::vector<uint32_t>> rows;
-            unsigned log_batch_max = 0;
-            for (auto& m : r.mats) {
-                heights.push_back(1ull << (m.log_n + log_blowup));
-                log_batch_max = std::max(log_batch_max, m.log_n + log_blowup);
-                std::vector<uint32_t> row(m.width);
-                for (auto& w : row) w = rd.fe();
-                rows.push_back(std::move(row));
-            }
-            if (log_batch_max > log_max) return "InvalidProofShape: matrix taller than the FRI domain";
-            std::vector<std::array<uint32_t, 8>> sib(log_batch_max);
-            for (auto& s : sib) rd.digest(s.data());
-            if (!rd.ok) return "InvalidProofShape: truncated query";
-            const uint64_t ridx = index >> (log_max - log_batch_max);
-            if (!verify_batch(r.commit, heights, rows, ridx, sib)) return "InvalidOpeningArgument:InputMmcsError";
-            for (size_t mi = 0; mi < r.mats.size(); mi++) {
-                const auto& m = r.mats[mi];
-                const unsigned lh = m.log_n + log_blowup;
-                const uint64_t rr = ridx >> (log_batch_max - lh);
-                const uint32_t x = kb::mul(gen, kb::pow(kb::two_adic_generator(lh), kb::bitrev((uint32_t)rr, lh)));
-                if (!ro.count(lh)) {
-                    ro[lh] = kb::ext_zero();
-                    apow[lh] = kb::ext_one();
-                }
-                for (size_t t = 0; t < m.points.size(); t++) {
-                    Ext d = kb::ext_neg(m.points[t]);
-                    d.c[0] = kb::add(d.c[0], x);  // x - z
-                    const Ext inv = kb::ext_inv(d);
-                    for (uint32_t c = 0; c < m.width; c++) {
-                        Ext diff = kb::ext_neg(m.values[t][c]);
-                        diff.c[0] = kb::add(diff.c[0], rows[mi][c]);  // p(x) - p(z)
-                        ro[lh] = kb::ext_add(ro[lh], kb::ext_mul(apow[lh], kb::ext_mul(diff, inv)));
-                        apow[lh] = kb::ext_mul(apow[lh], fri_alpha);
-                    }
-                }
-            }
-        }
-        // fold chain (fri/verifier.rs verify_query)
-        Ext folded = kb::ext_zero();
-        auto it = ro.begin();
-        uint64_t idx = index;
-        for (uint32_t k = 0; k < n_commit; k++) {
-            const unsigned lfh = log_max - 1 - k;
-            if (it != ro.end() && it->first == lfh + 1) {
-                // rolled in right after the fold of round k-1: plain, or scaled by that round's beta^2 (BFGPU_OPT_FRI_ROLLIN)
-                Ext r = it->second;
-                if (opt[BFGPU_OPT_FRI_ROLLIN] == 1 && k > 0) r = kb::ext_mul(kb::ext_sqr(betas[k - 1]), r);
-                folded = kb::ext_add(folded, r);
-                ++it;
-            }
-            Ext ev[2] = {folded, folded};
-            ev[(idx ^ 1) & 1] = rd.ext();
-            std::vector<std::array<uint32_t, 8>> sib(lfh);
-            for (auto& s : sib) rd.digest(s.data());
-            if (!rd.ok) return "InvalidProofShape: truncated commit-phase opening";
-            std::vector<uint32_t> row(8);
-            for (int e = 0; e < 2; e++)
-                for (int c = 0; c < 4; c++) row[4 * e + c] = ev[e].c[c];
-            if (!verify_batch(fri_commits[k].data(), {1ull << lfh}, {row}, idx >> 1, sib)) return "InvalidOpeningArgument:CommitPhaseMmcsError";
-            idx >>= 1;
-            // fold_row: e0 + (beta - x0) (e1 - e0) / (x1 - x0),  x0 = g_{lfh+1}^{bitrev(idx)}, x1 = -x0
-            const uint32_t x0 = kb::pow(kb::two_adic_generator(lfh + 1), kb::bitrev((uint32_t)idx, lfh));
-            Ext b = betas[k];
-            b.c[0] = kb::sub(b.c[0], x0);
-            const uint32_t den = kb::inv(kb::sub(kb::neg(x0), x0));
-            folded = kb::ext_add(ev[0], kb::ext_scale(kb::ext_mul(b, kb::ext_sub(ev[1], ev[0])), den));
-        }
-        if (it != ro.end()) return "InvalidOpeningArgument:InvalidProofShape";
-        if (!e_eq(folded, final_poly)) return "InvalidOpeningArgument:FinalPolyMismatch";
+        const uint64_t p = pl.q_base + q * pl.stride;
+        if (p < n_words && words[p] != pl.index[q]) pl.index_word_differs = true;
     }
-    if (index_word_differs) return "InvalidProofShape: query index";
-    if (rd.pos != rd.n) return "InvalidProofShape: trailing words";
-    // ---- constraints at zeta (verifier.rs:218-329) -----------------------------------------------------------------------------
+    pl.trailing = pl.stop_q == nq && pl.q_base + (uint64_t)nq * pl.stride != n_words;
+    return "";
+}
+
+// The first failing event of the query phase, in the order `verify` meets them.  Checks: input(q, r), commit(q, k) and
+// final_ok(q), called in exactly that order, each only after every earlier event of the walk has passed.
+template <class Checks>
+static std::string walk(const Plan& pl, Checks& ck) {
+    for (uint32_t q = 0; q < pl.nq_eff; q++) {
+        if (pl.stop_q == q && pl.stop_stage == 0) return "InvalidProofShape: truncated query";
+        for (int r = 0; r < 4; r++) {
+            if (pl.tall_round == r) return "InvalidProofShape: matrix taller than the FRI domain";
+            if (pl.stop_q == q && pl.stop_stage == 1u + r) return "InvalidProofShape: truncated query";
+            if (!ck.input(q, r)) return "InvalidOpeningArgument:InputMmcsError";
+        }
+        for (uint32_t k = 0; k < pl.n_commit; k++) {
+            if (pl.stop_q == q && pl.stop_stage == 5 + k) return "InvalidProofShape: truncated commit-phase opening";
+            if (!ck.commit(q, k)) return "InvalidOpeningArgument:CommitPhaseMmcsError";
+        }
+        if (pl.rollin_bad) return "InvalidOpeningArgument:InvalidProofShape";
+        if (!ck.final_ok(q)) return "InvalidOpeningArgument:FinalPolyMismatch";
+    }
+    if (pl.index_word_differs) return "InvalidProofShape: query index";
+    if (pl.trailing) return "InvalidProofShape: trailing words";
+    return "";
+}
+
+// Host executor of the plan: the per-query reduced openings (fri/two_adic_pcs.rs verify: open_input), MerkleTreeMmcs::verify_batch
+// and the fold chain (fri/verifier.rs verify_query), computed in the walk's order.
+struct HostChecks {
+    const Plan& pl;
+    const uint32_t* words;
+    std::map<unsigned, Ext, std::greater<unsigned>> ro;
+    std::map<unsigned, Ext> apow;
+    std::map<unsigned, Ext, std::greater<unsigned>>::iterator it;
+    Ext folded;
+    uint64_t idx = 0;
+    uint32_t fe(uint32_t q, uint64_t o) const {
+        const uint32_t v = words[pl.q_base + q * pl.stride + o];
+        return pl.monty ? v : kb::to_mont(v);
+    }
+    void digests(uint32_t q, uint64_t o, size_t n, std::vector<std::array<uint32_t, 8>>& out) const {
+        out.resize(n);
+        for (size_t l = 0; l < n; l++)
+            for (int j = 0; j < 8; j++) out[l][j] = fe(q, o + 8 * l + j);
+    }
+    bool input(uint32_t q, int r) {
+        if (r == 0) {
+            ro.clear();
+            apow.clear();
+        }
+        const unsigned log_blowup = pl.log_blowup, log_max = pl.log_max, log_batch_max = pl.round_lbm[r];
+        const auto& mats = pl.rounds[r].mats;
+        std::vector<uint64_t> heights;
+        std::vector<std::vector<uint32_t>> rows;
+        uint64_t o = pl.round_off[r];
+        for (auto& m : mats) {
+            heights.push_back(1ull << (m.log_n + log_blowup));
+            std::vector<uint32_t> row(m.width);
+            for (auto& w : row) w = fe(q, o++);
+            rows.push_back(std::move(row));
+        }
+        std::vector<std::array<uint32_t, 8>> sib;
+        digests(q, pl.sib_off[r], log_batch_max, sib);
+        const uint64_t ridx = pl.index[q] >> (log_max - log_batch_max);
+        if (!verify_batch(pl.rounds[r].commit, heights, rows, ridx, sib)) return false;
+        const uint32_t gen = kb::to_mont(kb::GEN);
+        for (size_t mi = 0; mi < mats.size(); mi++) {
+            const auto& m = mats[mi];
+            const unsigned lh = m.log_n + log_blowup;
+            const uint64_t rr = ridx >> (log_batch_max - lh);
+            const uint32_t x = kb::mul(gen, kb::pow(kb::two_adic_generator(lh), kb::bitrev((uint32_t)rr, lh)));
+            if (!ro.count(lh)) {
+                ro[lh] = kb::ext_zero();
+                apow[lh] = kb::ext_one();
+            }
+            for (size_t t = 0; t < m.points.size(); t++) {
+                Ext d = kb::ext_neg(m.points[t]);
+                d.c[0] = kb::add(d.c[0], x);  // x - z
+                const Ext inv = kb::ext_inv(d);
+                for (uint32_t c = 0; c < m.width; c++) {
+                    Ext diff = kb::ext_neg(m.values[t][c]);
+                    diff.c[0] = kb::add(diff.c[0], rows[mi][c]);  // p(x) - p(z)
+                    ro[lh] = kb::ext_add(ro[lh], kb::ext_mul(apow[lh], kb::ext_mul(diff, inv)));
+                    apow[lh] = kb::ext_mul(apow[lh], pl.fri_alpha);
+                }
+            }
+        }
+        if (r == 3) {
+            folded = kb::ext_zero();
+            it = ro.begin();
+            idx = pl.index[q];
+        }
+        return true;
+    }
+    bool commit(uint32_t q, uint32_t k) {
+        const unsigned lfh = pl.log_max - 1 - k;
+        if (it != ro.end() && it->first == lfh + 1) {
+            // rolled in right after the fold of round k-1: plain, or scaled by that round's beta^2 (BFGPU_OPT_FRI_ROLLIN)
+            Ext r = it->second;
+            if (pl.opt[BFGPU_OPT_FRI_ROLLIN] == 1 && k > 0) r = kb::ext_mul(kb::ext_sqr(pl.betas[k - 1]), r);
+            folded = kb::ext_add(folded, r);
+            ++it;
+        }
+        Ext ev[2] = {folded, folded};
+        for (int c = 0; c < 4; c++) ev[(idx ^ 1) & 1].c[c] = fe(q, pl.cp_off[k] + c);
+        std::vector<std::array<uint32_t, 8>> sib;
+        digests(q, pl.cp_off[k] + 4, lfh, sib);
+        std::vector<uint32_t> row(8);
+        for (int e = 0; e < 2; e++)
+            for (int c = 0; c < 4; c++) row[4 * e + c] = ev[e].c[c];
+        if (!verify_batch(pl.fri_commits[k].data(), {1ull << lfh}, {row}, idx >> 1, sib)) return false;
+        idx >>= 1;
+        // fold_row: e0 + (beta - x0) (e1 - e0) / (x1 - x0),  x0 = g_{lfh+1}^{bitrev(idx)}, x1 = -x0
+        const uint32_t x0 = kb::pow(kb::two_adic_generator(lfh + 1), kb::bitrev((uint32_t)idx, lfh));
+        Ext b = pl.betas[k];
+        b.c[0] = kb::sub(b.c[0], x0);
+        const uint32_t den = kb::inv(kb::sub(kb::neg(x0), x0));
+        folded = kb::ext_add(ev[0], kb::ext_scale(kb::ext_mul(b, kb::ext_sub(ev[1], ev[0])), den));
+        return true;
+    }
+    bool final_ok(uint32_t) const { return e_eq(folded, pl.final_poly); }
+};
+
+// ---- constraints at zeta (verifier.rs:218-329) -----------------------------------------------------------------------------
+static std::string constraints(const Plan& pl) {
+    const Round* rounds = pl.rounds;
+    const auto& chips = pl.chips;
+    const Ext zeta = pl.zeta;
+    const uint32_t gen = kb::to_mont(kb::GEN);
     size_t qpos = 0;
     std::map<int, size_t> prep_at;
-    for (size_t k = 0; k < prep.size(); k++) prep_at[prep[k].first] = k;
+    for (size_t k = 0; k < pl.prep.size(); k++) prep_at[pl.prep[k].first] = k;
     Ext total = kb::ext_zero();
     for (size_t i = 0; i < chips.size(); i++) {
         const auto& c = chips[i];
@@ -384,13 +523,13 @@ static std::string verify(const uint32_t vk_commit_in[8], const std::vector<std:
         R.perm0 = perm0.data();
         R.perm1 = perm1.data();
         air::Challenges chal;
-        chal.alpha = perm_ch[0];
+        chal.alpha = pl.perm_ch[0];
         chal.beta_pow[0] = kb::ext_one();
-        for (int k = 1; k < 8; k++) chal.beta_pow[k] = kb::ext_mul(chal.beta_pow[k - 1], perm_ch[1]);
+        for (int k = 1; k < 8; k++) chal.beta_pow[k] = kb::ext_mul(chal.beta_pow[k - 1], pl.perm_ch[1]);
         chal.cumulative_sum = c.csum;
         std::vector<Ext> apow(info.n_constraints);
         apow[0] = kb::ext_one();
-        for (int k = 1; k < info.n_constraints; k++) apow[k] = kb::ext_mul(apow[k - 1], alpha);
+        for (int k = 1; k < info.n_constraints; k++) apow[k] = kb::ext_mul(apow[k - 1], pl.alpha);
         Ext folded = kb::ext_zero();
         air::air_constraints_ext(c.chip, R, chal, apow.data(), folded);
         if (!e_eq(kb::ext_mul(folded, inv_zeroifier), quotient)) return fmt("OodEvaluationMismatch:%s", info.name);
@@ -400,58 +539,40 @@ static std::string verify(const uint32_t vk_commit_in[8], const std::vector<std:
     return "";
 }
 
+// returns "" when the proof is accepted, else the reference's error name (+ detail)
+static std::string verify(const uint32_t vk_commit[8], const std::vector<std::pair<int, unsigned>>& prep /* (chip index, log height), pk order */,
+                          const uint32_t* words, uint64_t n_words, bool monty, unsigned log_blowup, unsigned num_queries, unsigned pow_bits,
+                          const uint32_t opt[BFGPU_NUM_OPTS]) {
+    Plan pl;
+    std::string e = prepare(vk_commit, prep, words, n_words, monty, log_blowup, num_queries, pow_bits, opt, pl);
+    if (!e.empty()) return e;
+    HostChecks hc{pl, words};
+    e = walk(pl, hc);
+    return e.empty() ? constraints(pl) : e;
+}
+
 }  // namespace verifier
 
-// vk = preprocessed commitment + (chip name, log height) of every preprocessed trace in proving-key order.
-// repr: representation of vk_commit and of the proof words (BFGPU_REPR_*).  Returns BFGPU_OK when the proof is accepted;
-// otherwise BFGPU_ERR_INVALID with the reference's error name in `err`.
-extern "C" int32_t bfgpu_verify_shard_ex(const uint32_t vk_commit[8], const char* const* prep_names, const uint32_t* prep_log_heights, int32_t n_prep,
-                                         const uint32_t* proof, uint64_t n_words, int repr, uint32_t log_blowup, uint32_t num_queries, uint32_t pow_bits,
-                                         const uint32_t* options, int32_t n_options, char* err, uint64_t err_len) {
-    auto say = [&](const std::string& s) {
-        if (err && err_len) snprintf(err, (size_t)err_len, "%s", s.c_str());
-    };
-    if (!vk_commit || !proof || n_prep < 0 || (n_prep && (!prep_names || !prep_log_heights))) {
-        say("null argument");
-        return BFGPU_ERR_INVALID;
-    }
-    std::vector<std::pair<int, unsigned>> prep;
+namespace verifier {
+// (chip index, log height) of every preprocessed trace of the verifying key, pk order; "" or the entry points' argument error
+static std::string parse_prep(const char* const* prep_names, const uint32_t* prep_log_heights, int32_t n_prep, std::vector<std::pair<int, unsigned>>& prep) {
     for (int i = 0; i < n_prep; i++) {
         int ci = chip_index(prep_names[i]);
-        if (ci < 0) {
-            say(std::string("unknown chip ") + prep_names[i]);
-            return BFGPU_ERR_INVALID;
-        }
+        if (ci < 0) return std::string("unknown chip ") + prep_names[i];
         prep.emplace_back(ci, prep_log_heights[i]);
     }
-    uint32_t opt[BFGPU_NUM_OPTS] = {1, 0, 0};
+    return "";
+}
+static void parse_options(const uint32_t* options, int32_t n_options, uint32_t opt[BFGPU_NUM_OPTS]) {
+    opt[0] = 1, opt[1] = 0, opt[2] = 0;
     for (int32_t i = 0; options && i < n_options && i < BFGPU_NUM_OPTS; i++) opt[i] = options[i];
-    std::string e = verifier::verify(vk_commit, prep, proof, n_words, repr == BFGPU_REPR_MONTY, log_blowup, num_queries, pow_bits, opt);
-    say(e);
-    return e.empty() ? BFGPU_OK : BFGPU_ERR_INVALID;
 }
-extern "C" int32_t bfgpu_verify_shard(const uint32_t vk_commit[8], const char* const* prep_names, const uint32_t* prep_log_heights, int32_t n_prep,
-                                      const uint32_t* proof, uint64_t n_words, int repr, uint32_t log_blowup, uint32_t num_queries, uint32_t pow_bits,
-                                      char* err, uint64_t err_len) {
-    return bfgpu_verify_shard_ex(vk_commit, prep_names, prep_log_heights, n_prep, proof, n_words, repr, log_blowup, num_queries, pow_bits, nullptr, 0, err,
-                                 err_len);
-}
-
 // `BfProver::verify` (crates/prover/src/verify.rs:10-36) above `StarkMachine::verify` (crates/stark/src/machine.rs:258-284): the two
 // checks the reference makes on the proof before the shard verifier runs — the Cpu chip must be in `chip_ordering`
 // (MissingCpuInFirstShard) and its log degree must not exceed MAX_CPU_LOG_DEGREE = 22 (crates/core/machine/src/cpu/mod.rs:8: the LogUp
 // multiplicities must not overflow; CpuLogDegreeTooLarge) — then `verify_shard`, whose errors come back as "InvalidShardProof: ...".
-extern "C" int32_t bfgpu_verify_core_proof(const uint32_t vk_commit[8], const char* const* prep_names, const uint32_t* prep_log_heights, int32_t n_prep,
-                                           const uint32_t* proof, uint64_t n_words, int repr, uint32_t log_blowup, uint32_t num_queries, uint32_t pow_bits,
-                                           const uint32_t* options, int32_t n_options, char* err, uint64_t err_len) {
+static std::string core_precheck(const uint32_t* proof, uint64_t n_words) {
     constexpr uint32_t MAX_CPU_LOG_DEGREE = 22;
-    auto say = [&](const std::string& s) {
-        if (err && err_len) snprintf(err, (size_t)err_len, "%s", s.c_str());
-    };
-    if (!vk_commit || !proof) {
-        say("null argument");
-        return BFGPU_ERR_INVALID;
-    }
     // header of the serialisation: three commitments (24 words), the chip count, then (chip, log_degree, cumulative sum[4]) per chip
     const int cpu = chip_index("Cpu");
     const uint64_t n_chips = n_words > 24 ? proof[24] : 0;
@@ -462,18 +583,63 @@ extern "C" int32_t bfgpu_verify_core_proof(const uint32_t vk_commit[8], const ch
             has_cpu = true;
             log_degree_cpu = proof[25 + 6 * i + 1];
         }
-    if (!has_cpu) {
-        say("MissingCpuInFirstShard");
+    if (!has_cpu) return "MissingCpuInFirstShard";
+    if (log_degree_cpu > MAX_CPU_LOG_DEGREE) return fmt("CpuLogDegreeTooLarge: %u", log_degree_cpu);
+    return "";
+}
+// the shard verifier's error as bfgpu_verify_core_proof reports it (the inner message is held in a 256-byte buffer)
+static inline std::string core_wrap(const std::string& inner) { return inner.empty() ? inner : "InvalidShardProof: " + inner.substr(0, 255); }
+static void say(char* err, uint64_t err_len, const std::string& s) {
+    if (err && err_len) snprintf(err, (size_t)err_len, "%s", s.c_str());
+}
+}  // namespace verifier
+
+// vk = preprocessed commitment + (chip name, log height) of every preprocessed trace in proving-key order.
+// repr: representation of vk_commit and of the proof words (BFGPU_REPR_*).  Returns BFGPU_OK when the proof is accepted;
+// otherwise BFGPU_ERR_INVALID with the reference's error name in `err`.
+extern "C" int32_t bfgpu_verify_shard_ex(const uint32_t vk_commit[8], const char* const* prep_names, const uint32_t* prep_log_heights, int32_t n_prep,
+                                         const uint32_t* proof, uint64_t n_words, int repr, uint32_t log_blowup, uint32_t num_queries, uint32_t pow_bits,
+                                         const uint32_t* options, int32_t n_options, char* err, uint64_t err_len) {
+    if (!vk_commit || !proof || n_prep < 0 || (n_prep && (!prep_names || !prep_log_heights))) {
+        verifier::say(err, err_len, "null argument");
         return BFGPU_ERR_INVALID;
     }
-    if (log_degree_cpu > MAX_CPU_LOG_DEGREE) {
-        say(verifier::fmt("CpuLogDegreeTooLarge: %u", log_degree_cpu));
+    std::vector<std::pair<int, unsigned>> prep;
+    std::string e = verifier::parse_prep(prep_names, prep_log_heights, n_prep, prep);
+    if (!e.empty()) {
+        verifier::say(err, err_len, e);
+        return BFGPU_ERR_INVALID;
+    }
+    uint32_t opt[BFGPU_NUM_OPTS];
+    verifier::parse_options(options, n_options, opt);
+    e = verifier::verify(vk_commit, prep, proof, n_words, repr == BFGPU_REPR_MONTY, log_blowup, num_queries, pow_bits, opt);
+    verifier::say(err, err_len, e);
+    return e.empty() ? BFGPU_OK : BFGPU_ERR_INVALID;
+}
+extern "C" int32_t bfgpu_verify_shard(const uint32_t vk_commit[8], const char* const* prep_names, const uint32_t* prep_log_heights, int32_t n_prep,
+                                      const uint32_t* proof, uint64_t n_words, int repr, uint32_t log_blowup, uint32_t num_queries, uint32_t pow_bits,
+                                      char* err, uint64_t err_len) {
+    return bfgpu_verify_shard_ex(vk_commit, prep_names, prep_log_heights, n_prep, proof, n_words, repr, log_blowup, num_queries, pow_bits, nullptr, 0, err,
+                                 err_len);
+}
+
+// bfgpu_verify_shard_ex behind verifier::core_precheck (`BfProver::verify`)
+extern "C" int32_t bfgpu_verify_core_proof(const uint32_t vk_commit[8], const char* const* prep_names, const uint32_t* prep_log_heights, int32_t n_prep,
+                                           const uint32_t* proof, uint64_t n_words, int repr, uint32_t log_blowup, uint32_t num_queries, uint32_t pow_bits,
+                                           const uint32_t* options, int32_t n_options, char* err, uint64_t err_len) {
+    if (!vk_commit || !proof) {
+        verifier::say(err, err_len, "null argument");
+        return BFGPU_ERR_INVALID;
+    }
+    std::string e = verifier::core_precheck(proof, n_words);
+    if (!e.empty()) {
+        verifier::say(err, err_len, e);
         return BFGPU_ERR_INVALID;
     }
     char inner[256] = {0};
     int32_t rc = bfgpu_verify_shard_ex(vk_commit, prep_names, prep_log_heights, n_prep, proof, n_words, repr, log_blowup, num_queries, pow_bits, options,
                                        n_options, inner, sizeof inner);
-    say(rc == BFGPU_OK ? std::string() : std::string("InvalidShardProof: ") + inner);
+    verifier::say(err, err_len, rc == BFGPU_OK ? std::string() : std::string("InvalidShardProof: ") + inner);
     return rc;
 }
 
